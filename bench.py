@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this implementation (CUDA, C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # CPU port of the reference's path (oracle/)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
 Workload (config.workload): BASELINE.json configs[1] — synthetic 8k x 8k-nucleus embryo-like pair
 (N2 = 8000 fixed, N1 = 7200 moving after 10 % dropout, jitter 2 px), unsupervised
@@ -65,7 +66,14 @@ def parse():
     ap.add_argument("--no-square", action="store_true", help="skip the equal-counts (no slack columns) registration row")
     ap.add_argument("--lean", action="store_true",
                     help="profiling aid: warm-up + timed resident steps only (no e2e, stage, roofline or CPU legs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------------------------------- CPU arm
@@ -269,6 +277,34 @@ def bench_label_row(torch, D, hbm_peak, with_cpu):
 
 
 # ------------------------------------------------------------------------------------------- GPU arm
+DUMP_COST_ENTRIES = 1 << 20      # sampled entries per cost matrix: 4 x 4 MB of the ~25 MB a dump takes
+
+
+def dump_outputs(out_dir, res, cost, n1, n2):
+    """--dump-outputs: the results of one resident step as out_dir/<name>.npy, float64 (integers converted exactly)
+    or float32 (cost entries).  They are what a caller of register_described receives, copied to the host as the
+    public API copies them, and a fixed, seeded sample of the chi^2 cost matrices the step wrote into the caller's
+    buffer (`cost_sample` [hypothesis, k] at the flat row-major positions `cost_sample_index`).  lap_stats is left
+    out: it counts the solver's work, which may change between builds that compute the same results."""
+    import torch
+    from platymatch_b200.pipeline import _to_host
+    host = _to_host(res)
+    arrays = {k: np.asarray(host[k]) for k in ("transform", "transform_sc", "transform_icp", "ransac_A", "inliers",
+                                              "best", "lap_cost", "icp_residuals", "edge_ties")}
+    arrays["assignment_moving"] = np.stack([m for m, _ in host["assignments"]])
+    arrays["assignment_fixed"] = np.stack([f for _, f in host["assignments"]])
+    nr, nc = (n2, n1) if n1 > n2 else (n1, n2)
+    flat = np.unique(np.random.default_rng(0).integers(0, nr * nc, size=DUMP_COST_ENTRIES))
+    sel = torch.from_numpy(flat).to(cost.device)
+    arrays["cost_sample"] = cost[:, sel // nc, sel % nc].cpu().numpy()
+    arrays["cost_sample_index"] = flat
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.dtype != np.float32:
+            a = a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class ClockSampler:
     QUERY = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
              "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
@@ -591,11 +627,12 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms, what the last step returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for s in range(steps):
-            fn(s)
+            out = fn(s)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -603,16 +640,18 @@ def run_b200(args):
             t = torch.tensor([ms], dtype=torch.float64, device="cuda")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     for s in range(args.warmup):
         step_resident(s)
     torch.cuda.synchronize()
     sampler = ClockSampler(local) if rank == 0 else None
     l0 = lib.pm_launch_count()
-    ms = timed(step_resident, args.steps)
+    ms, last = timed(step_resident, args.steps)
     launches = lib.pm_launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, cost_buf, n1, n2)
     if args.lean:
         if rank == 0:
             print(json.dumps({"lean": True, "ms_per_step": ms / args.steps, "gpu_launches": int(launches)}), flush=True)
@@ -621,7 +660,7 @@ def run_b200(args):
         return
     for s in range(max(args.warmup, 3)):
         step_e2e(s)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     # ---- per-stage breakdown (CUDA events on the launching stream; stages serialised) ----
     marks = []

@@ -126,7 +126,7 @@ def counts_of(sc):
     return counts, totals
 
 
-def save_case(name, moving, fixed, res, trials, seed, full_cost=(0, 1), sub_rows=48, extra=None):
+def save_case(name, moving, fixed, res, trials, seed, sub_rows=16, picks=4000, extra=None):
     d = dict(moving=moving, fixed=fixed, trials=trials, seed=seed,
              moving_centroid=res["moving_centroid"], fixed_centroid=res["fixed_centroid"],
              moving_mean_distance=res["moving_mean_distance"], fixed_mean_distance=res["fixed_mean_distance"],
@@ -145,8 +145,10 @@ def save_case(name, moving, fixed, res, trials, seed, full_cost=(0, 1), sub_rows
         d["lap_cost_" + tag] = U[r, c].sum()
         d["cost_rowsum_" + tag], d["cost_colsum_" + tag] = U.sum(1), U.sum(0)
         d["cost_sub_" + tag] = U[:sub_rows]
-        if q in full_cost:
-            d["cost_full_" + tag] = U
+        # a seeded sample of the remaining entries instead of the whole matrix keeps the fixture under 1 MB
+        pool = np.arange(sub_rows * U.shape[1], U.size)
+        idx = np.sort(np.random.default_rng(q).choice(pool, min(picks, pool.size), replace=False)).astype(np.int32)
+        d["cost_pick_idx_" + tag], d["cost_pick_" + tag] = idx, U.ravel()[idx]
     if extra:
         d.update(extra)
     for k in ("kp_moving", "kp_fixed", "A_kp", "A_kp_icp"):
@@ -171,12 +173,12 @@ def main(which):
         m = load_asset("04-insitu.csv")
         f = REF.apply_affine_transform(m, A_GT_TEST)
         res = run_reference(m, f, trials=500, seed=1)
-        save_case("asset04", m, f, res, 500, 1, full_cost=(1,), sub_rows=16, extra=dict(A_gt=A_GT_TEST))
+        save_case("asset04", m, f, res, 500, 1, extra=dict(A_gt=A_GT_TEST))
     if "synth400" in which:  # rectangular, noisy: SURVEY §8d generator (jitter 2 px, 10 % dropout)
         from platymatch_b200.synthetic import make_pair, make_keypoints
         p = make_pair(400, seed=400)
         res = run_reference(p["moving"], p["fixed"], trials=1000, seed=2, keypoints=make_keypoints(p, 10, seed=3))
-        save_case("synth400", p["moving"], p["fixed"], res, 1000, 2, full_cost=(0, 1, 2, 3), sub_rows=16,
+        save_case("synth400", p["moving"], p["fixed"], res, 1000, 2,
                   extra=dict(A_gt=p["A_gt"], gt_fixed_index=p["gt_fixed_index"]))
 
 

@@ -119,22 +119,29 @@ def test_variants_are_phi_permutations(torch):
 
 
 # ------------------------------------------------------------------------------ K3
-def test_chi2_vs_reference_goldens(torch, golden):
-    """cost matrix within 1e-5 relative of the reference's float64 matrices."""
+def _unaries(get_unary, g):
+    um = get_unary(g["moving_centroid"], float(g["moving_mean_distance"]), g["moving"], "moving")
+    uf = get_unary(g["fixed_centroid"], float(g["fixed_mean_distance"]), g["fixed"], "fixed")
+    return {"u11": um[0], "u12": um[1], "u21": uf[0], "u22": uf[1], "u23": uf[2], "u24": uf[3]}
+
+
+def test_chi2_vs_reference_goldens(O, torch, golden):
+    """cost matrix within 1e-5 relative of the reference's float64 matrices: the rows and sampled entries the golden
+    keeps, and every entry of the oracle's matrix (pinned to the reference's by tests/test_oracle_golden.py)."""
     from platymatch_b200.estimate_transform.shape_context import unary_distance_matrix, get_unary
-    um = get_unary(golden["moving_centroid"], float(golden["moving_mean_distance"]), golden["moving"], "moving")
-    uf = get_unary(golden["fixed_centroid"], float(golden["fixed_mean_distance"]), golden["fixed"], "fixed")
-    u = {"u11": um[0], "u12": um[1], "u21": uf[0], "u22": uf[1], "u23": uf[2], "u24": uf[3]}
+    u, uo = _unaries(get_unary, golden), _unaries(O.get_unary, golden)
     worst = 0.0
     for tag in HYP_TAGS:
         ka, kb = UNARY_KEYS[tag]
         U = unary_distance_matrix(u[ka], u[kb])
         sub = golden["cost_sub_" + tag]
-        ref = golden["cost_full_" + tag] if "cost_full_" + tag in golden else sub
-        got = U[:ref.shape[0]]
-        nz = ref > 0
-        worst = max(worst, float((np.abs(got - ref)[nz] / ref[nz]).max()))
-        assert np.all(got[~nz] == 0.0)                      # identical histograms -> exactly 0, like the reference
+        checks = [(U[:sub.shape[0]], sub), (U, O.unary_distance_matrix(uo[ka], uo[kb]))]
+        if "cost_pick_" + tag in golden:
+            checks.append((U.ravel()[golden["cost_pick_idx_" + tag]], golden["cost_pick_" + tag]))
+        for got, ref in checks:
+            nz = ref > 0
+            worst = max(worst, float((np.abs(got - ref)[nz] / ref[nz]).max()))
+            assert np.all(got[~nz] == 0.0)                  # identical histograms -> exactly 0, like the reference
     assert worst < 1e-5, worst
 
 
@@ -246,11 +253,14 @@ def test_lap_sparse_auction_stats(O, torch):
 
 
 def test_lap_on_reference_cost_matrices(O, torch):
-    """The assignment scipy produced inside the reference run (golden) is reproduced on the same matrix."""
+    """The assignment scipy produced inside the reference run (golden) is reproduced on the same matrix: the oracle's,
+    which tests/test_oracle_golden.py pins to the reference's (it equals the reference's full matrices bit for bit)."""
     from platymatch_b200.lap import linear_sum_assignment
     g = load_golden("synth400")
+    u = _unaries(O.get_unary, g)
     for tag in ["11", "12", "13", "14"]:
-        U = g["cost_full_" + tag]
+        ka, kb = UNARY_KEYS[tag]
+        U = O.unary_distance_matrix(u[ka], u[kb])
         r, c = linear_sum_assignment(U)
         c32 = U.astype(np.float32).astype(np.float64)
         assert c32[r, c].sum() == pytest.approx(c32[g["lap_row_" + tag], g["lap_col_" + tag]].sum(), rel=1e-9)
