@@ -101,25 +101,16 @@ int pm_mean_distance(const double *pts, int n, double *out_mean, void *workspace
  * n_variants = 2 ('moving': sc, sc2) or 4 ('fixed': sc, sc2, sc3, sc4) or 1 (sc only).
  *   centroid   3 float64 (device)     x0  3 float64 (device)    mean_dist 1 float64 (device)
  *   r_edges    n_redges float64 (device) — numpy's logspace(log10(1/8), log10(2), 5) doubles
- *   counts     [n_variants][n][360] uint32  integer histograms (reference row = counts / row sum)
- *   dropped    [n_variants][n] uint32       neighbours not counted (overflow bins / NaN)
+ *   counts     [n_variants][rows][360] uint32  integer histograms (reference row = counts / row sum)
+ *   dropped    [n_variants][rows] uint32       neighbours not counted (overflow bins / NaN)
  *   edge_ties  [1] uint64, accumulated: neighbours whose r, theta or phi lies within 64 ulp of a
- *              bin edge (where another libm could decide differently); may be NULL. */
-int pm_shape_context_hist(const double *pts, int n, const double *centroid, const double *x0,
-                          const double *mean_dist, const double *r_edges, int n_redges, int n_variants,
-                          uint32_t *counts, uint32_t *dropped, unsigned long long *edge_ties, void *stream);
-
-/* The same for the query nuclei [row_begin, row_end) only (descriptor rows shard across GPUs, SURVEY §8e):
- * counts [n_variants][row_end - row_begin][360], dropped [n_variants][row_end - row_begin]. */
+ *              bin edge (where another libm could decide differently); may be NULL.
+ * Only the query nuclei [row_begin, row_end) are described, rows = row_end - row_begin (0, n for the whole
+ * cloud; descriptor rows shard across GPUs, SURVEY §8e). */
 int pm_shape_context_hist_rows(const double *pts, int n, const double *centroid, const double *x0,
                                const double *mean_dist, const double *r_edges, int n_redges, int n_variants,
                                int row_begin, int row_end, uint32_t *counts, uint32_t *dropped,
                                unsigned long long *edge_ties, void *stream);
-
-/* Normalise integer histograms (shape_context.py:41) to float32, written bin-major ("transposed"):
- * out[k * ld + i] = counts[i][k] / rowsum_i, ld >= n (pad columns hold zero_sentinel), exact zeros
- * replaced by zero_sentinel (0 keeps them).  Generic helper; the cost kernel uses pm_chi2_operand. */
-int pm_normalise_hist(const uint32_t *counts, int n, float *out, int ld, float zero_sentinel, void *stream);
 
 /* ---- K3  chi^2 histogram-distance cost matrix ---------------------------------------------------
  * get_unary_distance (shape_context.py:88-99) over all pairs (_dock_widget.py:547-602):
@@ -199,11 +190,6 @@ size_t pm_ransac_workspace_bytes(int trials);
 int pm_ransac(const double *moving, const double *fixed, int k, const int32_t *sample_idx, int trials, int min_samples,
               double error, unsigned long long seed, int transform, double *best_A, int32_t *best_inliers,
               int32_t *best_trial, int32_t *inliers_per_trial, void *workspace, size_t workspace_bytes, void *stream);
-/* = pm_ransac(..., PM_TRANSFORM_AFFINE, ...) */
-int pm_ransac_affine(const double *moving, const double *fixed, int k, const int32_t *sample_idx, int trials,
-                     int min_samples, double error, unsigned long long seed, double *best_A,
-                     int32_t *best_inliers, int32_t *best_trial, int32_t *inliers_per_trial, void *workspace,
-                     size_t workspace_bytes, void *stream);
 
 /* ---- K6  ICP with affine re-fit -------------------------------------------------------------------
  * perform_icp (perform_icp.py:7-26): `iterations` x { nearest fixed point per moving point (first
@@ -212,15 +198,13 @@ int pm_ransac_affine(const double *moving, const double *fixed, int k, const int
  *   moving [n1][3] float64 — NOT modified;  fixed [n2][3] float64
  *   A_icp [16] float64 out; residuals [iterations] float64 out (mean ||moving' - fixed[nn]||,
  *   get_error utils.py:77-88), may be NULL;  nn_out [n1] int32 last nearest-neighbour map, may be NULL.
- * workspace: pm_icp_workspace_bytes(n1). */
-size_t pm_icp_workspace_bytes(int n1);            /* brute-force nearest neighbour only */
-size_t pm_icp_workspace_bytes2(int n1, int n2);  /* + the uniform grid over the fixed cloud (exact, ~50x fewer candidates) */
+ * Nearest neighbours come from a uniform grid over the fixed cloud (exact, ~50x fewer candidates); fewer than 256
+ * fixed points are searched by brute force.
+ * workspace: pm_icp_workspace_bytes2(n1, n2), else PM_ERR_WORKSPACE. */
+size_t pm_icp_workspace_bytes2(int n1, int n2);
 /* perform_icp with its `transform` argument (re-fit = get_affine_transform or get_similar_transform, :17-20) */
 int pm_icp(const double *moving, int n1, const double *fixed, int n2, int iterations, int transform, double *A_icp,
            double *residuals, int32_t *nn_out, void *workspace, size_t workspace_bytes, void *stream);
-/* = pm_icp(..., PM_TRANSFORM_AFFINE, ...) */
-int pm_icp_affine(const double *moving, int n1, const double *fixed, int n2, int iterations, double *A_icp,
-                  double *residuals, int32_t *nn_out, void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- small ops -------------------------------------------------------------------------------------
  * get_affine_transform (find_transform.py:4-17) = fixed_h @ pinv(moving_h) for K >= 1 pairs: float64 normal

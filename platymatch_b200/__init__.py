@@ -14,7 +14,7 @@ plus the fused pipeline (`estimate_transform_unsupervised`, `estimate_transform_
 `EstimateTransform._click_run` (_dock_widget.py:526-721).  Hand-written CUDA behind a C ABI
 (include/platymatch_b200.h, platymatch_b200/csrc); no CPU fallback.
 """
-__version__ = "0.1.0"
+__version__ = "0.2.0"
 
 from ._lib import load as load_library, LIB_PATH, PlatyMatchError  # noqa: F401
 

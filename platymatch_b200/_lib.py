@@ -32,9 +32,7 @@ SIGNATURES = {
     "pm_cloud_stats": (_i, [_vp, _i, _vp, _vp]),
     "pm_mean_distance_workspace_bytes": (_sz, [_i]),
     "pm_mean_distance": (_i, [_vp, _i, _vp, _vp, _sz, _vp]),
-    "pm_shape_context_hist": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "pm_shape_context_hist_rows": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
-    "pm_normalise_hist": (_i, [_vp, _i, _vp, _i, ctypes.c_float, _vp]),
     "pm_chi2_operand": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "pm_chi2_operand_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "pm_chi2_cost": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _i, _vp]),
@@ -42,11 +40,8 @@ SIGNATURES = {
     "pm_lap_solve": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pm_ransac_workspace_bytes": (_sz, [_i]),
     "pm_ransac": (_i, [_vp, _vp, _i, _vp, _i, _i, _d, _u64, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "pm_ransac_affine": (_i, [_vp, _vp, _i, _vp, _i, _i, _d, _u64, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "pm_icp_workspace_bytes": (_sz, [_i]),
     "pm_icp_workspace_bytes2": (_sz, [_i, _i]),
     "pm_icp": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "pm_icp_affine": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pm_fit_affine": (_i, [_vp, _vp, _i, _vp, _vp]),
     "pm_fit_similar": (_i, [_vp, _vp, _i, _vp, _vp]),
     "pm_select_best": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),

@@ -13,7 +13,7 @@ void pm_set_error(const char *fmt, ...) {
     va_end(ap);
 }
 
-extern "C" int pm_version(void) { return 100; /* 0.1.0 */ }
+extern "C" int pm_version(void) { return 200; /* 0.2.0 */ }
 extern "C" const char *pm_last_error_string(void) { return g_pm_error; }
 
 extern "C" int pm_device_count(void) {

@@ -53,9 +53,9 @@ extern "C" int pm_host_shape_context(const double *pts, int n, const double *cen
     PM_CUDA_TRY(cudaMemcpy(dsmall.p, small, sizeof(small), cudaMemcpyHostToDevice));
     PM_TRY(pm_cloud_stats(dpts.as<double>(), n, dstats.as<double>(), 0));
     double *ds = dsmall.as<double>();
-    PM_TRY(pm_shape_context_hist(dpts.as<double>(), n, ds, dstats.as<double>() + 3, ds + 3, ds + 4, n_redges,
-                                 n_variants, dcounts.as<uint32_t>(), ddropped.as<uint32_t>(),
-                                 reinterpret_cast<unsigned long long *>(ds + 10), 0));
+    PM_TRY(pm_shape_context_hist_rows(dpts.as<double>(), n, ds, dstats.as<double>() + 3, ds + 3, ds + 4, n_redges,
+                                      n_variants, 0, n, dcounts.as<uint32_t>(), ddropped.as<uint32_t>(),
+                                      reinterpret_cast<unsigned long long *>(ds + 10), 0));
     PM_CUDA_TRY(cudaMemcpy(counts, dcounts.p, cbytes, cudaMemcpyDeviceToHost));
     if (dropped)
         PM_CUDA_TRY(cudaMemcpy(dropped, ddropped.p, (size_t)n_variants * n * sizeof(uint32_t), cudaMemcpyDeviceToHost));

@@ -590,26 +590,42 @@ static int pm_icp_grid_target(int n2) {      // cells along the longest axis: ~2
     return t;
 }
 
-static size_t pm_icp_grid_bytes(int n2) {
-    const size_t t = (size_t)pm_icp_grid_target(n2) + 1, max_cells = t * t * t;
-    return pm_align256(sizeof(PmIcpGrid)) + 2 * pm_align256((max_cells + 1) * sizeof(int))   // cell_start, cursor
-         + pm_align256((size_t)n2 * sizeof(int)) * 2                                          // cell_of, sorted_idx
-         + pm_align256((size_t)n2 * 3 * sizeof(double));                                      // sorted_pts
+static size_t pm_icp_max_cells(int n2) {
+    const size_t t = (size_t)pm_icp_grid_target(n2) + 1;
+    return t * t * t;
+}
+
+// byte offsets of the workspace of pm_icp, and its total size
+struct PmIcpLayout {
+    size_t cur, nn, partial, small, res_partial, grid, cell_start, cursor, cell_of, sorted_idx, sorted_pts, total;
+};
+
+static PmIcpLayout pm_icp_layout(int n1, int n2) {
+    const size_t nb_nn = (size_t)(n1 + PM_ICP_PTS - 1) / PM_ICP_PTS;
+    const size_t nb_res = (size_t)(n1 + PM_ICP_QPB - 1) / PM_ICP_QPB;
+    const size_t max_cells = pm_icp_max_cells(n2);
+    PmIcpLayout L;
+    size_t o = 0;
+    L.cur = o; o += pm_align256((size_t)n1 * 3 * sizeof(double));
+    L.nn = o; o += pm_align256((size_t)n1 * sizeof(int32_t));
+    L.partial = o; o += pm_align256((nb_nn + 2 * nb_res) * PM_ICP_NSUM * sizeof(double));   // ping-pong for the persistent kernel
+    L.small = o; o += pm_align256(64 * sizeof(double));                                     // a_est, a_icp, shift
+    L.res_partial = o; o += pm_align256(nb_res * sizeof(double) * 1024);                   // residual partials (<= 1024 iterations)
+    // uniform grid over the fixed cloud
+    L.grid = o; o += pm_align256(sizeof(PmIcpGrid));
+    L.cell_start = o; o += pm_align256((max_cells + 1) * sizeof(int));
+    L.cursor = o; o += pm_align256((max_cells + 1) * sizeof(int));
+    L.cell_of = o; o += pm_align256((size_t)n2 * sizeof(int));
+    L.sorted_idx = o; o += pm_align256((size_t)n2 * sizeof(int));
+    L.sorted_pts = o; o += pm_align256((size_t)n2 * 3 * sizeof(double));
+    L.total = o;
+    return L;
 }
 
 extern "C" size_t pm_icp_workspace_bytes2(int n1, int n2) {
     if (n1 < 1 || n2 < 1) return 0;
-    const size_t nb_nn = (size_t)(n1 + PM_ICP_PTS - 1) / PM_ICP_PTS;
-    const size_t nb_res = (size_t)(n1 + PM_ICP_QPB - 1) / PM_ICP_QPB;
-    return pm_align256((size_t)n1 * 3 * sizeof(double))          // cur
-         + pm_align256((size_t)n1 * sizeof(int32_t))             // nn
-         + pm_align256((nb_nn + 2 * nb_res) * PM_ICP_NSUM * sizeof(double))     // partial (ping-pong for the persistent kernel)
-         + pm_align256(64 * sizeof(double))                      // a_est, a_icp, shift
-         + pm_align256(nb_res * sizeof(double) * 1024)           // residual partials (<= 1024 iterations)
-         + pm_icp_grid_bytes(n2);                                // uniform grid over the fixed cloud
+    return pm_icp_layout(n1, n2).total;
 }
-
-extern "C" size_t pm_icp_workspace_bytes(int n1) { return pm_icp_workspace_bytes2(n1, 0 + 1) - pm_icp_grid_bytes(1); }
 
 extern "C" int pm_icp(const double *moving, int n1, const double *fixed, int n2, int iterations, int transform,
                       double *A_icp, double *residuals, int32_t *nn_out, void *workspace, size_t workspace_bytes,
@@ -618,34 +634,30 @@ extern "C" int pm_icp(const double *moving, int n1, const double *fixed, int n2,
     PM_REQUIRE(n1 >= 1 && n2 >= 1, "need n1 >= 1 and n2 >= 1");
     PM_REQUIRE(transform == PM_TRANSFORM_AFFINE || transform == PM_TRANSFORM_SIMILAR, "unknown transform");
     PM_REQUIRE(iterations >= 0 && iterations <= 1024, "iterations must be 0..1024");
-    if (workspace_bytes < pm_icp_workspace_bytes(n1)) {
+    const PmIcpLayout L = pm_icp_layout(n1, n2);
+    if (workspace_bytes < L.total) {
         pm_set_error("pm_icp: workspace too small");
         return PM_ERR_WORKSPACE;
     }
-    // the grid search needs the larger workspace of pm_icp_workspace_bytes2 (and pays off from a few hundred points)
-    const bool use_grid = n2 >= 256 && workspace_bytes >= pm_icp_workspace_bytes2(n1, n2) && !getenv("PM_ICP_BRUTE");
+    // the grid search pays off from a few hundred fixed points
+    const bool use_grid = n2 >= 256 && !getenv("PM_ICP_BRUTE");
     cudaStream_t s = pm_stream(stream);
     const int nb_nn = (n1 + PM_ICP_PTS - 1) / PM_ICP_PTS, nb_ap = (n1 + 255) / 256;
-    char *w = (char *)workspace;
-    double *cur = (double *)w; w += pm_align256((size_t)n1 * 3 * sizeof(double));
-    int32_t *nn = (int32_t *)w; w += pm_align256((size_t)n1 * sizeof(int32_t));
     const int nb_pers = (n1 + PM_ICP_QPB - 1) / PM_ICP_QPB;
-    double *partial = (double *)w; w += pm_align256((size_t)(nb_nn + 2 * nb_pers) * PM_ICP_NSUM * sizeof(double));
-    double *small = (double *)w; w += pm_align256(64 * sizeof(double));
-    double *res_partial = (double *)w; w += pm_align256((size_t)nb_pers * sizeof(double) * 1024);
+    char *w = (char *)workspace;
+    double *cur = (double *)(w + L.cur);
+    int32_t *nn = (int32_t *)(w + L.nn);
+    double *partial = (double *)(w + L.partial);
+    double *small = (double *)(w + L.small);
+    double *res_partial = (double *)(w + L.res_partial);
     double *a_est = small, *a_icp = small + 16, *shift = small + 32;
-    PmIcpGrid *grid = nullptr;
-    int *cell_start = nullptr, *cursor = nullptr, *cell_of = nullptr, *sorted_idx = nullptr;
-    double *sorted_pts = nullptr;
+    PmIcpGrid *grid = (PmIcpGrid *)(w + L.grid);
+    int *cell_start = (int *)(w + L.cell_start), *cursor = (int *)(w + L.cursor);
+    int *cell_of = (int *)(w + L.cell_of), *sorted_idx = (int *)(w + L.sorted_idx);
+    double *sorted_pts = (double *)(w + L.sorted_pts);
     if (use_grid) {
-        const size_t t = (size_t)pm_icp_grid_target(n2) + 1, max_cells = t * t * t;
-        grid = (PmIcpGrid *)w; w += pm_align256(sizeof(PmIcpGrid));
-        cell_start = (int *)w; w += pm_align256((max_cells + 1) * sizeof(int));
-        cursor = (int *)w; w += pm_align256((max_cells + 1) * sizeof(int));
-        cell_of = (int *)w; w += pm_align256((size_t)n2 * sizeof(int));
-        sorted_idx = (int *)w; w += pm_align256((size_t)n2 * sizeof(int));
-        sorted_pts = (double *)w;
-        pm_icp_grid_setup_kernel<<<1, 1024, 0, s>>>(fixed, n2, pm_icp_grid_target(n2), grid, cell_start, (int)max_cells);
+        pm_icp_grid_setup_kernel<<<1, 1024, 0, s>>>(fixed, n2, pm_icp_grid_target(n2), grid, cell_start,
+                                                    (int)pm_icp_max_cells(n2));
         pm_icp_cell_count_kernel<<<(n2 + 255) / 256, 256, 0, s>>>(fixed, n2, grid, cell_of, cell_start);
         pm_icp_cell_scan_kernel<<<1, 1024, 0, s>>>(grid, cell_start, cursor);
         pm_icp_cell_fill_kernel<<<(n2 + 255) / 256, 256, 0, s>>>(fixed, n2, cell_of, cursor, sorted_pts, sorted_idx);
@@ -696,11 +708,4 @@ extern "C" int pm_icp(const double *moving, int n1, const double *fixed, int n2,
     if (nn_out && iterations > 0)
         PM_CUDA_TRY(cudaMemcpyAsync(nn_out, nn, (size_t)n1 * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
     return PM_OK;
-}
-
-extern "C" int pm_icp_affine(const double *moving, int n1, const double *fixed, int n2, int iterations,
-                             double *A_icp, double *residuals, int32_t *nn_out, void *workspace,
-                             size_t workspace_bytes, void *stream) {
-    return pm_icp(moving, n1, fixed, n2, iterations, PM_TRANSFORM_AFFINE, A_icp, residuals, nn_out, workspace,
-                  workspace_bytes, stream);
 }

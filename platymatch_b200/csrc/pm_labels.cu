@@ -305,126 +305,6 @@ __global__ void __launch_bounds__(256, 3) pm_label_stream_kernel(const T *__rest
     }
 }
 
-// ---- the same pass with the volume staged by the bulk-copy engine ----------------------------------------------
-// The register-staged kernel above is latency-bound (ncu: 7.9 long-scoreboard stalls per issue, DRAM at 65 % of its
-// peak): what a warp can keep in flight is what its registers hold.  Here every warp owns a ring of PM_LABEL_TMA_STAGES
-// 4 KB shared-memory buffers that the copy engine fills (`cp.async.bulk.shared::cluster.global` + mbarrier
-// complete_tx; SASS: UBLKCP / SYNCS): 12 KB per warp, 96 KB per CTA, 192 KB per SM in flight without a register.
-// One lane arms a buffer's barrier with the byte count and issues the copy; all lanes wait on the barrier's phase,
-// read their chunks (lane-contiguous 16-byte loads, conflict-free), and after a __syncwarp the buffer is re-armed with
-// the block PM_LABEL_TMA_STAGES further on.  No CTA-wide synchronisation after the barrier initialisation.
-// RESULT (round 2, one B200): bit-identical tables (tests/test_labels.py passes with it as the default), but 86 us
-// against 77 us for the register-staged kernel: with 4 KB per copy and 16 warps per SM the examine loop of a warp and
-// its copies do not overlap as well as 24 warps with loads in registers do.  Kept opt-in (PM_LABEL_TMA=1) as the
-// starting point for larger blocks per copy / a dedicated producer warp.
-#define PM_LABEL_TMA_STAGES 3
-#define PM_LABEL_TMA_CHUNKS 256          // 16-byte chunks per block: 8 per lane, 4 KB
-
-__device__ __forceinline__ bool pm_mbar_try_wait(unsigned addr, unsigned parity) {
-    unsigned ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(addr), "r"(parity) : "memory");
-    return ok != 0u;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(256, 2) pm_label_tma_kernel(const T *__restrict__ labels, int nz, int ny, int nx,
-                                                           unsigned table_size, unsigned long long *__restrict__ acc) {
-    constexpr int VPC = 16 / (int)sizeof(T);
-    extern __shared__ __align__(128) unsigned char pm_label_smem[];
-    // dynamic: [8 warps][STAGES][256] uint4 | [8][STAGES] mbarrier (u64)
-    uint4 *s_buf = reinterpret_cast<uint4 *>(pm_label_smem);
-    unsigned long long *s_bar = reinterpret_cast<unsigned long long *>(s_buf + 8 * PM_LABEL_TMA_STAGES * PM_LABEL_TMA_CHUNKS);
-    __shared__ uint4 s_q[8][PM_LABEL_QCAP];
-    __shared__ unsigned s_c[8][PM_LABEL_QCAP];
-    const size_t n_vox = (size_t)nz * ny * nx;
-    const size_t n_chunks = n_vox / VPC;
-    const size_t n_blocks = (n_chunks + PM_LABEL_TMA_CHUNKS - 1) / PM_LABEL_TMA_CHUNKS;
-    const unsigned plane = (unsigned)ny * (unsigned)nx;
-    const uint4 *__restrict__ p = reinterpret_cast<const uint4 *>(labels);
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const unsigned lt = (1u << lane) - 1u;
-    const size_t n_warps = (size_t)gridDim.x * 8, warp_id = (size_t)blockIdx.x * 8 + w;
-    uint4 *my_buf = s_buf + (size_t)w * PM_LABEL_TMA_STAGES * PM_LABEL_TMA_CHUNKS;
-    const unsigned bar0 = (unsigned)__cvta_generic_to_shared(s_bar + w * PM_LABEL_TMA_STAGES);
-    const unsigned buf0 = (unsigned)__cvta_generic_to_shared(my_buf);
-    if (lane == 0) {
-#pragma unroll
-        for (int st = 0; st < PM_LABEL_TMA_STAGES; ++st)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar0 + 8u * st) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    auto issue = [&](int st, size_t blk) {          // lane 0: arm the barrier with the byte count, start the copy
-        const size_t c0 = blk * PM_LABEL_TMA_CHUNKS;
-        const size_t left = n_chunks - c0;
-        const unsigned bytes = (unsigned)((left < PM_LABEL_TMA_CHUNKS ? left : (size_t)PM_LABEL_TMA_CHUNKS) * 16);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar0 + 8u * st), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     :: "r"(buf0 + (unsigned)st * (PM_LABEL_TMA_CHUNKS * 16)), "l"(p + c0), "r"(bytes), "r"(bar0 + 8u * st) : "memory");
-    };
-    int queued = 0;                                              // warp-uniform
-    auto flush = [&]() {
-        __syncwarp();
-        for (int i = lane; i < queued; i += 32)
-            pm_label_chunk<T>(s_q[w][i], (size_t)s_c[w][i] * VPC, plane, (unsigned)ny, (unsigned)nx, table_size, acc);
-        queued = 0;
-        __syncwarp();
-    };
-    if (lane == 0) {
-#pragma unroll
-        for (int st = 0; st < PM_LABEL_TMA_STAGES; ++st) {
-            const size_t blk = warp_id + (size_t)st * n_warps;
-            if (blk < n_blocks) issue(st, blk);
-        }
-    }
-    int st = 0;
-    unsigned parity = 0;
-    for (size_t blk = warp_id; blk < n_blocks; blk += n_warps) {
-        unsigned spins = 0;
-        while (!pm_mbar_try_wait(bar0 + 8u * st, parity))
-            if (++spins > (1u << 28)) __trap();                  // (a lost copy must not hang the GPU)
-        const size_t c0 = blk * PM_LABEL_TMA_CHUNKS;
-        const uint4 *buf = my_buf + (size_t)st * PM_LABEL_TMA_CHUNKS;
-#pragma unroll
-        for (int u = 0; u < PM_LABEL_TMA_CHUNKS / 32; ++u) {
-            const size_t idx = c0 + (size_t)u * 32 + lane;
-            uint4 q = buf[u * 32 + lane];
-            if (!(idx < n_chunks)) q = make_uint4(0u, 0u, 0u, 0u);      // (beyond the last chunk: stale bytes of the ring)
-            const bool fg = (q.x | q.y | q.z | q.w) != 0u;
-            const unsigned bal = __ballot_sync(0xffffffffu, fg);
-            if (bal) {
-                if (queued + __popc(bal) > PM_LABEL_QCAP) flush();
-                if (fg) {
-                    const int pos = queued + __popc(bal & lt);
-                    s_q[w][pos] = q;
-                    s_c[w][pos] = (unsigned)idx;
-                }
-                queued += __popc(bal);
-            }
-        }
-        __syncwarp();                                            // every lane has read the buffer: refill it
-        const size_t nxt = blk + (size_t)PM_LABEL_TMA_STAGES * n_warps;
-        if (lane == 0 && nxt < n_blocks) issue(st, nxt);
-        if (queued >= 32) flush();
-        if (++st == PM_LABEL_TMA_STAGES) { st = 0; parity ^= 1u; }
-    }
-    flush();
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-        for (size_t v = n_chunks * VPC; v < n_vox; ++v) {         // < VPC voxels
-            const int id = (int)labels[v];
-            if (id > 0 && (unsigned)id < table_size) {
-                const unsigned pz = (unsigned)(v / plane), rem = (unsigned)(v - (size_t)pz * plane);
-                unsigned long long *a = acc + (size_t)id * 4;
-                atomicAdd(a + 0, 1ull);
-                atomicAdd(a + 1, (unsigned long long)pz);
-                atomicAdd(a + 2, (unsigned long long)(rem / nx));
-                atomicAdd(a + 3, (unsigned long long)(rem % nx));
-            }
-        }
-    }
-}
-
 // ids with a non-zero count, ascending (np.unique order), -> ids / centroids (z, y, x) / sizes.
 // One CTA per 1024 ids, one id per thread: the three float64 divisions per nucleus and the loads of its sums spread
 // over as many SMs as there are chunks (one CTA doing all of it took 19-36 us for 6000 ids, a quarter of the whole
@@ -499,20 +379,7 @@ static int pm_label_run(const T *labels, int nz, int ny, int nx, unsigned table_
     const int blocks = (int)(want < (size_t)sms * 8 ? (want ? want : 1) : (size_t)sms * 8);   // 8 resident CTAs per SM
     const bool stream_ok = (reinterpret_cast<size_t>(labels) & 15) == 0 && (size_t)ny * nx < ((size_t)1 << 32) &&
                            n_vox / (16 / sizeof(T)) < ((size_t)1 << 32) && !getenv("PM_LABEL_WARP_KERNEL");
-    if (stream_ok && getenv("PM_LABEL_TMA")) {
-        // bulk-copy staged kernel: 2 CTAs per SM (96 KB of staging each), one wave.  Opt-in: measured 86 us against
-        // 77 us for the register-staged kernel on the 403 MB bench volume (profiles/r2_label_tma_experiment.txt)
-        const size_t smem = (size_t)8 * PM_LABEL_TMA_STAGES * PM_LABEL_TMA_CHUNKS * 16 + 8 * PM_LABEL_TMA_STAGES * 8;
-        static int tma_ready[64];                                  // per device: attribute raised (benign race)
-        if (!(dev >= 0 && dev < 64) || !tma_ready[dev]) {
-            PM_CUDA_TRY(cudaFuncSetAttribute(pm_label_tma_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (dev >= 0 && dev < 64) tma_ready[dev] = 1;
-        }
-        const size_t chunks = n_vox / (16 / sizeof(T));
-        size_t want3 = (chunks + 8 * PM_LABEL_TMA_CHUNKS - 1) / (8 * PM_LABEL_TMA_CHUNKS);
-        const int blocks3 = (int)(want3 < (size_t)sms * 2 ? (want3 ? want3 : 1) : (size_t)sms * 2);
-        pm_label_tma_kernel<T><<<blocks3, 256, smem, s>>>(labels, nz, ny, nx, table_size, acc);
-    } else if (stream_ok) {
+    if (stream_ok) {
         // ONE wave of resident CTAs (the kernel is a grid-stride loop): no second wave that starts ragged
         const size_t chunks = n_vox / (16 / sizeof(T));
         static int occ_cache[64];                                  // per device (benign race: every writer stores the same value)

@@ -32,6 +32,13 @@ namespace cg = cooperative_groups;
 
 // squared (dummy rows + eps-scaling) when nc - nr <= this fraction of nc; measured crossover at 8k, profiles/r2_lap_slack.txt
 #define PM_LAP_SQUARE_SLACK_DEFAULT 0.02
+// eps-scaling schedule of a squared problem (DESIGN §4 K4): the first eps is this fraction of the matrix' cost scale,
+// divided by PM_LAP_EPS_THETA from phase to phase, over PM_LAP_EPS_PHASES phases
+#define PM_LAP_EPS0 (1.0 / 16.0)
+#define PM_LAP_EPS_THETA 8.0
+#define PM_LAP_EPS_PHASES 6
+// an eps phase stops carrying displaced rows once this few warps are still bidding; measured, profiles/r2_lap_eps_truncation.txt
+#define PM_LAP_EPS_STOP_LIVE 3
 #define PM_LAP_BID_THREADS 1024
 #define PM_LAP_CPT 8
 #define PM_LAP_MAX_THREADS 1024
@@ -124,7 +131,6 @@ struct PmLapBatch {   // passed by value to kernels
     int ring_in_smem;
     // eps-scaling phases (problems without slack columns): increment = certified gap + eps, eps = eps_factor x the
     // matrix' own cost scale (mean candidate-list width, accumulated by pm_ls_build_lists into scale[0..1] per matrix)
-    int dummies_bid;     // tail kernel: dummy rows take part (0 in the early eps phases: they stay free there)
     double eps_factor;   // 0 = exact phase (eps = 0)
     double *scale;       // [batch][2]: sum of list widths, number of rows that contributed
 };
@@ -807,7 +813,7 @@ __global__ void __launch_bounds__(1024, 1) pm_ls_auction_kernel(PmLapBatch B) {
     __syncthreads();
     for (int base = 0; base < nr; base += blockDim.x) {
         const int i = base + t;
-        const bool is_free = (i < nr) && (V.col4row[i] < 0) && (B.dummies_bid || i < B.nr_real);
+        const bool is_free = (i < nr) && (V.col4row[i] < 0);
         const unsigned bal = __ballot_sync(0xffffffffu, is_free);
         if (lane == 0) s_scan[t >> 5] = __popc(bal);
         __syncthreads();
@@ -1526,11 +1532,9 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
     // (see below).  The dummies take the columns that stay unassigned, so the optimum over the real rows is the same.
     bool square = false;
     if (max_bid_rounds > 0 && algorithm != PM_LAP_ALGO_DENSE_AUCTION && nr >= 64) {
-        double max_slack = PM_LAP_SQUARE_SLACK_DEFAULT;        // of nc; above it the pure epsilon = 0 schedule is faster
-        const char *e = getenv("PM_LAP_SQUARE_SLACK");
-        if (e) max_slack = atof(e);
-        square = (double)(nc - nr) <= max_slack * (double)nc;
-        e = getenv("PM_LAP_EPS_SCALING");
+        // above this slack the pure epsilon = 0 schedule is faster
+        square = (double)(nc - nr) <= PM_LAP_SQUARE_SLACK_DEFAULT * (double)nc;
+        const char *e = getenv("PM_LAP_EPS_SCALING");
         if (e) square = atoi(e) != 0;
     }
     if (square) B.nr = nc;
@@ -1539,7 +1543,6 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
     B.scale = (double *)((char *)workspace + 256);
     B.zero_row = (const float *)((char *)workspace + 256 + pm_lap_align((size_t)batch * 2 * sizeof(double)));
     B.eps_factor = 0.0;
-    B.dummies_bid = 1;
     B.ws = (char *)workspace + pm_lap_header_bytes(batch, B.ncp);
     B.col4row = col4row; B.stats = (long long *)stats; B.total = total;
     // one "round" of the sparse auction = a budget of one bid per row, spread over the 32 warps
@@ -1606,49 +1609,27 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
         // tight edges as the warm start of the exact (epsilon = 0) phase + augmenting paths below, so the result is
         // the exact optimum as before.  (With slack columns the prices of columns that end up unassigned would have
         // to return to zero, which eps-scaling cannot guarantee: those keep the pure epsilon = 0 schedule.)
-        const bool eps_scaling = square;
-        if (eps_scaling) {
-            double factor = 1.0 / 16.0, theta = 8.0;
-            int phases = 6;
-            const char *e = getenv("PM_LAP_EPS0");
-            if (e && atof(e) > 0.0) factor = atof(e);
-            e = getenv("PM_LAP_EPS_THETA");
-            if (e && atof(e) > 1.0) theta = atof(e);
-            e = getenv("PM_LAP_EPS_PHASES");
-            if (e && atoi(e) > 0) phases = atoi(e);
+        if (square) {
             // The end of an eps phase is a handful of chains that fight sequentially (measured at 8000 x 8000: bulk
             // kernel 4.0 / 0.8 / 0.4 ms, then 54 / 31 / 14 ms of ONE CTA finishing phases 1-3 to the last row).  The phases
-            // only prepare prices (exactness comes from the finish below), so they are TRUNCATED: the early ones end
-            // when the bulk kernel's parallelism has collapsed, the last `tail_phases` ones also run the tail kernel
-            // (where the dummies bid), which stops carrying displaced rows once `eps_stop` warps are left.
-            int tail_phases = phases, eps_stop = 3, eps_stop_last = 3;   // measured: profiles/r2_lap_eps_truncation.txt
-            e = getenv("PM_LAP_EPS_TAIL_PHASES");
-            if (e && atoi(e) > 0) tail_phases = atoi(e);
-            e = getenv("PM_LAP_EPS_STOP_LIVE");
-            if (e && atoi(e) >= 0) eps_stop = atoi(e);
-            e = getenv("PM_LAP_EPS_STOP_LAST");
-            if (e && atoi(e) >= 0) eps_stop_last = atoi(e);
-            int dummy_phases = phases;                        // the dummies bid in the last `dummy_phases` eps phases
-            e = getenv("PM_LAP_EPS_DUMMY_PHASES");
-            if (e && atoi(e) >= 0) dummy_phases = atoi(e);
+            // only prepare prices (exactness comes from the finish below), so they are TRUNCATED: the bulk kernel ends
+            // when its parallelism has collapsed, and the tail kernel (where the dummies bid) stops carrying displaced
+            // rows once PM_LAP_EPS_STOP_LIVE warps are left.
             const int stop_live = B.stop_live;
-            for (int k = 0; k < phases; ++k, factor /= theta) {
+            B.stop_live = PM_LAP_EPS_STOP_LIVE;
+            double factor = PM_LAP_EPS0;
+            for (int k = 0; k < PM_LAP_EPS_PHASES; ++k, factor /= PM_LAP_EPS_THETA) {
                 B.eps_factor = factor;
-                B.stop_live = (k == phases - 1) ? eps_stop_last : eps_stop;
-                B.dummies_bid = k >= phases - dummy_phases;
                 if (k > 0) {
                     pm_ls_phase_reset_kernel<<<dim3(32, batch), 256, 0, s>>>(B);
                     PM_LAUNCH_CHECK();
                 }
                 pm_ls_bulk_kernel<<<batch * bulk_ctas, 256, 0, s>>>(B, bulk_ctas);
                 PM_LAUNCH_CHECK();
-                if (k >= phases - tail_phases) {
-                    pm_ls_auction_kernel<<<batch, 1024, tail_smem, s>>>(B);
-                    PM_LAUNCH_CHECK();
-                }
+                pm_ls_auction_kernel<<<batch, 1024, tail_smem, s>>>(B);
+                PM_LAUNCH_CHECK();
             }
             B.eps_factor = 0.0;
-            B.dummies_bid = 1;
             B.stop_live = stop_live;
             if (B.nr > B.nr_real) {
                 pm_ls_equalise_dummies_kernel<<<batch, 1024, 0, s>>>(B);
@@ -1676,8 +1657,7 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
     }
     int rc;
     const size_t ss_smem = (size_t)B.ncp * (8 + 8 + 2 + 2 + 2 + 1);
-    if (max_bid_rounds > 0 && algorithm == PM_LAP_ALGO_SPARSE_AUCTION && ss_smem + 2048 <= (size_t)smem_optin &&
-        !getenv("PM_LAP_DENSE_SAP")) {
+    if (max_bid_rounds > 0 && algorithm == PM_LAP_ALGO_SPARSE_AUCTION && ss_smem + 2048 <= (size_t)smem_optin) {
         if (int rc = pm_lap_raise_smem_limit(pm_lap_sap_sparse_kernel, smem_optin, dev)) return rc;
         pm_lap_sap_sparse_kernel<<<batch, PM_SS_THREADS, ss_smem, s>>>(B);
         PM_LAUNCH_CHECK();

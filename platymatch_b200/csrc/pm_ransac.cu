@@ -243,11 +243,3 @@ extern "C" int pm_ransac(const double *moving, const double *fixed, int k, const
     PM_LAUNCH_CHECK();
     return PM_OK;
 }
-
-extern "C" int pm_ransac_affine(const double *moving, const double *fixed, int k, const int32_t *sample_idx,
-                                int trials, int min_samples, double error, unsigned long long seed, double *best_A,
-                                int32_t *best_inliers, int32_t *best_trial, int32_t *inliers_per_trial,
-                                void *workspace, size_t workspace_bytes, void *stream) {
-    return pm_ransac(moving, fixed, k, sample_idx, trials, min_samples, error, seed, PM_TRANSFORM_AFFINE, best_A,
-                     best_inliers, best_trial, inliers_per_trial, workspace, workspace_bytes, stream);
-}

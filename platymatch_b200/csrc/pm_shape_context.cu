@@ -266,57 +266,3 @@ extern "C" int pm_shape_context_hist_rows(const double *pts, int n, const double
     PM_LAUNCH_CHECK();
     return PM_OK;
 }
-
-extern "C" int pm_shape_context_hist(const double *pts, int n, const double *centroid, const double *x0,
-                                     const double *mean_dist, const double *r_edges, int n_redges,
-                                     int n_variants, uint32_t *counts, uint32_t *dropped,
-                                     unsigned long long *edge_ties, void *stream) {
-    return pm_shape_context_hist_rows(pts, n, centroid, x0, mean_dist, r_edges, n_redges, n_variants, 0, n, counts,
-                                      dropped, edge_ties, stream);
-}
-
-// Normalise to float32, bin-major (coalesced operand layout of the chi^2 kernel).
-// grid: (ceil(ld/32), ceil(360/32)), block 32x8: tiled transpose through shared memory.
-__global__ void __launch_bounds__(256) pm_normalise_hist_kernel(const uint32_t *__restrict__ counts, int n,
-                                                                float *__restrict__ out, int ld,
-                                                                float zero_sentinel) {
-    __shared__ float tile[32][33];
-    __shared__ float inv_total[32];
-    const int i0 = blockIdx.x * 32, k0 = blockIdx.y * 32;
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // ty 0..7
-    // row totals for the 32 nuclei of this tile: warp ty handles rows ty, ty+8, ...
-    for (int r = ty; r < 32; r += 8) {
-        const int i = i0 + r;
-        uint32_t s = 0;
-        if (i < n)
-            for (int k = tx; k < PM_NBINS; k += 32) s += counts[(size_t)i * PM_NBINS + k];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        if (tx == 0) inv_total[r] = (float)s;
-    }
-    __syncthreads();
-    for (int r = ty; r < 32; r += 8) {
-        const int i = i0 + r, k = k0 + tx;
-        float v = zero_sentinel;   // pad columns (i >= n) behave like empty bins
-        if (i < n && k < PM_NBINS) {
-            const uint32_t c = counts[(size_t)i * PM_NBINS + k];
-            v = (c == 0u) ? zero_sentinel : (float)c / inv_total[r];   // count / total, one rounding
-        }
-        tile[r][tx] = v;
-    }
-    __syncthreads();
-    for (int r = ty; r < 32; r += 8) {
-        const int k = k0 + r, i = i0 + tx;
-        if (k < PM_NBINS && i < ld) out[(size_t)k * ld + i] = tile[tx][r];
-    }
-}
-
-extern "C" int pm_normalise_hist(const uint32_t *counts, int n, float *out, int ld, float zero_sentinel,
-                                 void *stream) {
-    PM_REQUIRE(counts && out, "null pointer");
-    PM_REQUIRE(n >= 1 && ld >= n, "need n >= 1 and ld >= n");
-    dim3 grid((ld + 31) / 32, (PM_NBINS + 31) / 32);
-    pm_normalise_hist_kernel<<<grid, 256, 0, pm_stream(stream)>>>(counts, n, out, ld, zero_sentinel);
-    PM_LAUNCH_CHECK();
-    return PM_OK;
-}

@@ -80,17 +80,6 @@ def padded(n, tile=CHI2_TILE):
     return ((n + tile - 1) // tile) * tile
 
 
-def normalise(counts_2d, zero_sentinel=0.0):
-    """[N,360] counts -> bin-major float32 [360, ld] (ld = N rounded up to 128); generic helper."""
-    torch = _torch()
-    n = counts_2d.shape[0]
-    ld = padded(n)
-    out = torch.empty((NBINS, ld), dtype=torch.float32, device=counts_2d.device)
-    check(load().pm_normalise_hist(ptr(counts_2d), n, ptr(out), ld, float(zero_sentinel), stream_ptr()),
-          "pm_normalise_hist")
-    return out
-
-
 class Chi2Operand:
     """One side of the chi^2 cost kernel: bin-major float32 histograms [361, ld] (empty bins = 2^-60, row
     360 = null bin) and the per-128-block non-empty-bin masks [ld/128, 12] (see pm_chi2_operand)."""
@@ -184,10 +173,6 @@ def ransac(moving_k, fixed_k, trials, error, min_samples=4, sample_idx=None, see
     return best_a, best_inl, best_trial, per_trial
 
 
-def ransac_affine(moving_k, fixed_k, trials, error, min_samples=4, sample_idx=None, seed=0, want_per_trial=False):
-    return ransac(moving_k, fixed_k, trials, error, min_samples, sample_idx, seed, want_per_trial, 'Affine')
-
-
 def icp(moving, fixed, iterations=50, want_nn=False, transform='Affine'):
     """-> (A_icp [16] f64, residuals [iterations] f64, nn [N1] i32 | None)."""
     torch = _torch()
@@ -200,10 +185,6 @@ def icp(moving, fixed, iterations=50, want_nn=False, transform='Affine'):
     check(load().pm_icp(ptr(moving), n1, ptr(fixed), n2, int(iterations), transform_code(transform), ptr(a_icp),
                         ptr(resid), ptr(nn), ptr(ws), nbytes, stream_ptr()), "pm_icp")
     return a_icp, resid[:iterations], nn
-
-
-def icp_affine(moving, fixed, iterations=50, want_nn=False):
-    return icp(moving, fixed, iterations, want_nn, 'Affine')
 
 
 def fit_transform(moving_k, fixed_k, transform='Affine'):
@@ -226,10 +207,6 @@ def select_best(inliers, a_all):
     a = torch.empty(16, dtype=torch.float64, device=inliers.device)
     check(load().pm_select_best(ptr(inliers), ptr(a_all), n, ptr(best), ptr(a), stream_ptr()), "pm_select_best")
     return best, a
-
-
-def fit_affine(moving_k, fixed_k):
-    return fit_transform(moving_k, fixed_k, 'Affine')
 
 
 def apply_affine(pts, a16):

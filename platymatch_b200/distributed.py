@@ -18,7 +18,7 @@ Three ways the path shards:
                         all-gather (`allgather_counts`); cost rows are delivered to the matrix OWNER ONLY: on NCCL
                         the chi^2 kernel stores them straight into the owner's matrix through a peer-mapped window
                         (device.PeerWindow, CUDA IPC over NVLink: compute and transfer are one kernel), otherwise
-                        (gloo, or PM_DIST_NO_PEER=1) with one `dist.gather` per matrix (`gather_rows_to_owner`).
+                        (gloo, or peer_stores=False) with one `dist.gather` per matrix (`gather_rows_to_owner`).
                         The LAP itself does not shard across GPUs ("replicas only"): one matrix, one GPU.
 
 The partition arithmetic and the exchange steps are plain-tensor code (CPU or CUDA), covered by world_size-2
@@ -26,7 +26,6 @@ gloo tests in tests/test_distributed_cpu.py; `register_pair_sharded` and `regist
 library and are covered by tests/test_gpu_distributed.py (torchrun, NCCL, 2 GPUs).
 """
 import itertools
-import os
 import collections
 import threading
 import time
@@ -296,7 +295,7 @@ def register_pair_sharded(moving, fixed, *, ransac_samples=4, ransac_trials=8000
     need_m, need_f = max(a for a, _ in hyps), max(b for _, b in hyps)
     nccl = world > 1 and dist.get_backend(group) == "nccl"
     if peer_stores is None:
-        peer_stores = nccl and not os.environ.get("PM_DIST_NO_PEER")
+        peer_stores = nccl
 
     def mark(name, t0):
         if timings is not None:

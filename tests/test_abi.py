@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import shutil
+import subprocess
 
 import pytest
 
@@ -23,6 +25,12 @@ def test_header_symbols_exported_and_bound():
         assert hasattr(lib, n), "missing export " + n
         assert n in _lib.SIGNATURES, "no ctypes signature for " + n
     assert set(_lib.SIGNATURES) == set(names)
+    # and the library exports nothing else: a definition left behind by a removed declaration shows up here
+    nm = shutil.which("nm")
+    if nm:
+        out = subprocess.run([nm, "-D", "--defined-only", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+        exported = {f[-1] for f in (line.split() for line in out.splitlines()) if f and f[-1].startswith("pm_")}
+        assert exported == set(names), (sorted(exported - set(names)), sorted(set(names) - exported))
 
 
 def test_ctypes_signatures_match_header_arity():
@@ -38,14 +46,14 @@ def test_ctypes_signatures_match_header_arity():
         assert n == len(_lib.SIGNATURES[name][1]), (name, n, len(_lib.SIGNATURES[name][1]))
 
 
-def test_version_and_sizes_without_gpu():
+def test_version_and_workspace_sizes_without_gpu():
     from platymatch_b200 import _lib
     lib = _lib.load()
-    assert lib.pm_version() == 100
+    assert lib.pm_version() == 200
     assert lib.pm_mean_distance_workspace_bytes(8000) == 32 * 32 * 8
     assert lib.pm_lap_workspace_bytes(4, 7200, 8000) > 4 * (7200 + 8000) * 8
     assert lib.pm_ransac_workspace_bytes(8000) >= 8000 * 13 * 8
-    assert lib.pm_icp_workspace_bytes(7200) >= 7200 * 24
+    assert lib.pm_icp_workspace_bytes2(7200, 8000) >= 7200 * 24 + 8000 * 24
     assert isinstance(lib.pm_last_error_string(), bytes)
 
 

@@ -118,6 +118,37 @@ def test_variants_are_phi_permutations(torch):
     assert np.array_equal(h[3][:, :, (5 - k) % 12], h[0])
 
 
+def test_host_entry_points_match_device_path(torch):
+    """pm_host_mean_distance / pm_host_shape_context (the numpy callers' entry points, INTEGRATION.md §2) return
+    exactly what get_mean_distance / get_unary_counts return."""
+    import ctypes
+    from platymatch_b200 import _lib
+    from platymatch_b200.device import R_EDGES
+    from platymatch_b200.estimate_transform.shape_context import get_unary_counts
+    from platymatch_b200.utils.utils import get_mean_distance
+    lib, vp = _lib.load(), ctypes.c_void_p
+    g = load_golden("asset02")
+    pts = np.ascontiguousarray(g["fixed"].T[:, :3], dtype=np.float64)
+    n = pts.shape[0]
+    md = ctypes.c_double()
+    _lib.check(lib.pm_host_mean_distance(pts.ctypes.data_as(vp), n, 0, ctypes.byref(md)), "pm_host_mean_distance")
+    assert md.value == get_mean_distance(g["fixed"], transposed=False)
+    c = np.ascontiguousarray(g["fixed_centroid"], dtype=np.float64).reshape(-1)[:3]
+    mean_dist = float(g["fixed_mean_distance"])
+    edges = np.ascontiguousarray(R_EDGES, dtype=np.float64)
+    counts = np.empty((4, n, 360), dtype=np.uint32)
+    dropped = np.empty((4, n), dtype=np.uint32)
+    x0 = np.empty(3, dtype=np.float64)
+    ties = ctypes.c_ulonglong()
+    _lib.check(lib.pm_host_shape_context(pts.ctypes.data_as(vp), n, c.ctypes.data_as(vp), mean_dist,
+                                         edges.ctypes.data_as(vp), edges.size, 4, 0, counts.ctypes.data_as(vp),
+                                         dropped.ctypes.data_as(vp), x0.ctypes.data_as(vp), ctypes.byref(ties)),
+               "pm_host_shape_context")
+    d_counts, d_dropped, d_ties, d_x0 = get_unary_counts(c, mean_dist, g["fixed"], "fixed")
+    assert np.array_equal(counts, d_counts) and np.array_equal(dropped, d_dropped)
+    assert np.array_equal(x0, d_x0) and ties.value == d_ties
+
+
 # ------------------------------------------------------------------------------ K3
 def _unaries(get_unary, g):
     um = get_unary(g["moving_centroid"], float(g["moving_mean_distance"]), g["moving"], "moving")
@@ -296,28 +327,28 @@ def test_ransac_vs_reference_goldens(O, torch, golden):
         assert np.allclose(A, golden["ransac_A"][q], rtol=1e-7, atol=1e-7), tag
 
 
-def test_ransac_per_trial_counts_and_device_rng(O, D, torch):
+def test_ransac_affine_per_trial_counts_and_device_rng(O, D, torch):
     p = _pair(800, seed=8)
     k = p["moving"].shape[1]
     m, f = p["moving"], p["fixed"][:, p["gt_fixed_index"]]
     idx = O.ransac_sample_indices(k, 4, 300, seed=4)
     _, _, inl_o, mats = O.do_ransac(m, f, 4, 300, 16, sample_indices=idx, return_all=True)
     md, fd = D.to_device_points(m), D.to_device_points(f)
-    a, inl, trial, per = D.ransac_affine(md, fd, 300, 16.0, 4, torch.from_numpy(idx).cuda(), want_per_trial=True)
+    a, inl, trial, per = D.ransac(md, fd, 300, 16.0, 4, torch.from_numpy(idx).cuda(), want_per_trial=True)
     assert np.array_equal(per.cpu().numpy(), inl_o)
     assert trial.item() == int(np.argmax(inl_o))
     # device Philox sampling: deterministic per seed, indices distinct, finds the true affine on clean matches
-    a1, i1, _, _ = D.ransac_affine(md, fd, 500, 16.0, 4, None, seed=123)
-    a2, i2, _, _ = D.ransac_affine(md, fd, 500, 16.0, 4, None, seed=123)
+    a1, i1, _, _ = D.ransac(md, fd, 500, 16.0, 4, None, seed=123)
+    a2, i2, _, _ = D.ransac(md, fd, 500, 16.0, 4, None, seed=123)
     assert i1.item() == i2.item() and torch.equal(a1, a2) and i1.item() > 0.9 * k
     # no inliers at all (negative threshold) -> all-ones matrix and 0, as the reference (shape_context.py:120)
-    a0, i0, t0, _ = D.ransac_affine(md, fd, 20, -1.0, 4, None, seed=1)
+    a0, i0, t0, _ = D.ransac(md, fd, 20, -1.0, 4, None, seed=1)
     assert i0.item() == 0 and torch.all(a0 == 1.0) and t0.item() == -1
     # coplanar (degenerate) samples: numpy's pinv still answers (minimum-norm affine), so does the kernel; never NaN
     mflat = m.copy(); mflat[2] = 5.0
     idx3 = O.ransac_sample_indices(k, 4, 50, seed=2)
     _, i3_o, per3_o, _ = O.do_ransac(mflat, f, 4, 50, 16, sample_indices=idx3, return_all=True)
-    a3, i3, _, per3 = D.ransac_affine(D.to_device_points(mflat), fd, 50, 16.0, 4, torch.from_numpy(idx3).cuda(), want_per_trial=True)
+    a3, i3, _, per3 = D.ransac(D.to_device_points(mflat), fd, 50, 16.0, 4, torch.from_numpy(idx3).cuda(), want_per_trial=True)
     assert i3.item() == i3_o and np.array_equal(per3.cpu().numpy(), per3_o) and torch.all(torch.isfinite(a3))
 
 
@@ -332,16 +363,16 @@ def test_icp_vs_reference_goldens(torch, golden):
     assert np.abs(a_icp @ golden["A_sc"] - golden["A_final"]).max() < 1e-4
 
 
-def test_icp_nearest_neighbour_map(O, D, torch):
+def test_icp_affine_nearest_neighbour_map(O, D, torch):
     p = _pair(1500, seed=2)
     m = O.apply_affine_transform(p["moving"], p["A_gt"])
-    _, _, nn = D.icp_affine(D.to_device_points(m), D.to_device_points(p["fixed"]), 1, want_nn=True)
+    _, _, nn = D.icp(D.to_device_points(m), D.to_device_points(p["fixed"]), 1, want_nn=True)
     nn_o, _ = O.nearest(m, p["fixed"])
     assert np.array_equal(nn.cpu().numpy(), nn_o)
 
 
 @pytest.mark.parametrize("case", ["shell", "filled", "outliers", "lattice_ties", "identical", "flat"])
-def test_icp_grid_search_matches_brute_force(O, D, torch, case, monkeypatch):
+def test_icp_affine_grid_search_matches_brute_force(O, D, torch, case, monkeypatch):
     """The uniform-grid search returns exactly the brute-force nearest-neighbour map (first minimum in ascending
     index), also with exact distance ties, queries far outside the fixed cloud's box and degenerate boxes."""
     rng = np.random.default_rng(len(case))
@@ -358,16 +389,16 @@ def test_icp_grid_search_matches_brute_force(O, D, torch, case, monkeypatch):
         f = rng.random((3, 1200)) * 50; m = f[:, rng.permutation(1200)[:900]].copy()
     else:
         f = rng.random((3, 1000)) * 80; f[0] = 7.0; m = rng.random((3, 700)) * 80          # zero extent along z
-    _, _, nn = D.icp_affine(D.to_device_points(m), D.to_device_points(f), 1, want_nn=True)
+    _, _, nn = D.icp(D.to_device_points(m), D.to_device_points(f), 1, want_nn=True)
     nn_o, _ = O.nearest(m, f)
     assert np.array_equal(nn.cpu().numpy(), nn_o)
     monkeypatch.setenv("PM_ICP_BRUTE", "1")
-    a_b, r_b, nn_b = D.icp_affine(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
+    a_b, r_b, nn_b = D.icp(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
     monkeypatch.delenv("PM_ICP_BRUTE")
     monkeypatch.setenv("PM_ICP_MULTI_LAUNCH", "1")          # grid search, three launches per iteration
-    a_g, r_g, nn_g = D.icp_affine(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
+    a_g, r_g, nn_g = D.icp(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
     monkeypatch.delenv("PM_ICP_MULTI_LAUNCH")               # grid search, whole loop in one cooperative launch
-    a_p, r_p, nn_p = D.icp_affine(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
+    a_p, r_p, nn_p = D.icp(D.to_device_points(m), D.to_device_points(f), 3, want_nn=True)
     assert torch.equal(nn_b, nn_g) and torch.equal(nn_b, nn_p)
     if case != "lattice_ties":                               # (there the fit is rank deficient: NaN rows)
         assert torch.allclose(a_b, a_g, rtol=1e-9, atol=1e-9, equal_nan=True)
