@@ -165,6 +165,17 @@ int pm_chi2_cost(const float *a_t, int lda, const uint32_t *a_mask, int n1, cons
 #define PM_LAP_STAT_AUCTION_CYCLES 10 /* sparse auction: SM cycles of the longest-running warp */
 #define PM_LAP_STAT_BULK_BIDS 11      /* sparse auction: bids made by the multi-SM bulk kernel */
 #define PM_LAP_STAT_SAP_DENSE_RELAX 12 /* sparse augmenting paths: tree rows that had to be relaxed densely */
+#define PM_LAP_STAT_PATH 13           /* kernels this solve ran: PM_LAP_PATH_* bits */
+/* path bits: squared with dummy rows; the auction that ran (neither bit: max_bid_rounds = 0, augmenting paths only);
+ * exactly one finishing kernel; the sparse auction's ring of displaced rows in shared memory (else global memory) */
+#define PM_LAP_PATH_SQUARED 1
+#define PM_LAP_PATH_SPARSE_AUCTION 2
+#define PM_LAP_PATH_DENSE_AUCTION 4
+#define PM_LAP_PATH_SAP_SPARSE 8   /* augmenting paths over the candidate lists (pm_lap_sap_sparse_kernel) */
+#define PM_LAP_PATH_SAP_DENSE8 16  /* dense augmenting paths, 8 columns per thread, prices in registers */
+#define PM_LAP_PATH_SAP_DENSE16 32 /* dense augmenting paths, 16 columns per thread */
+#define PM_LAP_PATH_SAP_DENSE24 64 /* dense augmenting paths, 24 columns per thread */
+#define PM_LAP_PATH_RING_SMEM 128
 #define PM_LAP_ALGO_AUTO 0
 #define PM_LAP_ALGO_SPARSE_AUCTION 1
 #define PM_LAP_ALGO_DENSE_AUCTION 2

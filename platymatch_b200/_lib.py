@@ -11,6 +11,9 @@ LIB_PATH = os.path.join(_HERE, "libplatymatch_b200.so")
 
 NBINS = 360
 LAP_STATS = 16
+# PM_LAP_PATH_* bits of the assignment's `path` statistic (PM_LAP_STAT_PATH): which kernels a solve ran
+LAP_PATH = {"SQUARED": 1, "SPARSE_AUCTION": 2, "DENSE_AUCTION": 4, "SAP_SPARSE": 8, "SAP_DENSE8": 16,
+            "SAP_DENSE16": 32, "SAP_DENSE24": 64, "RING_SMEM": 128}
 CHI2_EPS = 2.0 ** -60
 CHI2_TILE = 128
 TRANSFORMS = {"Affine": 0, "Similar": 1}      # PM_TRANSFORM_* (the widget's strings, _dock_widget.py:627)

@@ -133,6 +133,7 @@ struct PmLapBatch {   // passed by value to kernels
     // matrix' own cost scale (mean candidate-list width, accumulated by pm_ls_build_lists into scale[0..1] per matrix)
     double eps_factor;   // 0 = exact phase (eps = 0)
     double *scale;       // [batch][2]: sum of list widths, number of rows that contributed
+    int path;            // PM_LAP_PATH_* bits of this solve, reported by the finishing kernel as PM_LAP_STAT_PATH
 };
 
 // cost row of row i (dummy rows share one row of zeros)
@@ -1238,6 +1239,7 @@ __global__ void __launch_bounds__(PM_LAP_MAX_THREADS, 1) pm_lap_sap_kernel(PmLap
             V.stats[PM_LAP_STAT_AUGMENTATIONS] = nfree;
             V.stats[PM_LAP_STAT_DIJKSTRA_STEPS] = steps;
             V.stats[PM_LAP_STAT_STATUS] = status;
+            V.stats[PM_LAP_STAT_PATH] = B.path;
         }
     }
     (void)final_parity;
@@ -1453,6 +1455,7 @@ __global__ void __launch_bounds__(PM_SS_THREADS, 1) pm_lap_sap_sparse_kernel(PmL
             V.stats[PM_LAP_STAT_DIJKSTRA_STEPS] = steps;
             V.stats[PM_LAP_STAT_STATUS] = status;
             V.stats[PM_LAP_STAT_SAP_DENSE_RELAX] = dense_relax;
+            V.stats[PM_LAP_STAT_PATH] = B.path;
         }
     }
 }
@@ -1584,6 +1587,11 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
     }
     if (algorithm == PM_LAP_ALGO_AUTO) algorithm = sparse_fits ? PM_LAP_ALGO_SPARSE_AUCTION : PM_LAP_ALGO_DENSE_AUCTION;
     if (algorithm != PM_LAP_ALGO_SPARSE_AUCTION && square) { square = false; B.nr = nr; }   // (only the sparse auction bids for dummy rows)
+    B.path = square ? PM_LAP_PATH_SQUARED : 0;
+    if (max_bid_rounds > 0)
+        B.path |= algorithm == PM_LAP_ALGO_SPARSE_AUCTION
+                      ? PM_LAP_PATH_SPARSE_AUCTION | (B.ring_in_smem ? PM_LAP_PATH_RING_SMEM : 0)
+                      : PM_LAP_PATH_DENSE_AUCTION;
 
     pm_lap_init_kernel<<<dim3(32, batch), 256, 0, s>>>(B);
     PM_LAUNCH_CHECK();
@@ -1659,6 +1667,7 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
     const size_t ss_smem = (size_t)B.ncp * (8 + 8 + 2 + 2 + 2 + 1);
     if (max_bid_rounds > 0 && algorithm == PM_LAP_ALGO_SPARSE_AUCTION && ss_smem + 2048 <= (size_t)smem_optin) {
         if (int rc = pm_lap_raise_smem_limit(pm_lap_sap_sparse_kernel, smem_optin, dev)) return rc;
+        B.path |= PM_LAP_PATH_SAP_SPARSE;
         pm_lap_sap_sparse_kernel<<<batch, PM_SS_THREADS, ss_smem, s>>>(B);
         PM_LAUNCH_CHECK();
         rc = PM_OK;
@@ -1666,10 +1675,13 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
         int threads = ((nc + PM_LAP_CPT - 1) / PM_LAP_CPT + 31) & ~31;
         if (threads < 64) threads = 64;
         if (threads > PM_LAP_MAX_THREADS) threads = PM_LAP_MAX_THREADS;
+        B.path |= PM_LAP_PATH_SAP_DENSE8;
         rc = pm_lap_launch_sap<PM_LAP_CPT, true>(B, batch, threads, smem_optin, dev, s);
     } else if (nc <= 16 * PM_LAP_MAX_THREADS) {
+        B.path |= PM_LAP_PATH_SAP_DENSE16;
         rc = pm_lap_launch_sap<16, false>(B, batch, PM_LAP_MAX_THREADS, smem_optin, dev, s);
     } else {
+        B.path |= PM_LAP_PATH_SAP_DENSE24;
         rc = pm_lap_launch_sap<24, false>(B, batch, PM_LAP_MAX_THREADS, smem_optin, dev, s);
     }
     return rc;

@@ -13,6 +13,8 @@ def linear_sum_assignment(cost_matrix, maximize=False, return_stats=False, max_b
     The matrix is solved as float32 values with float64 duals (optimal for the float32-rounded
     matrix).  Tall matrices are solved through the transpose, as scipy does.
     algorithm: 0 auto, 1 sparse asynchronous auction, 2 dense grid-wide auction (PM_LAP_ALGO_*).
+    return_stats adds the solver's statistics; `path` holds the PM_LAP_PATH_* bits of the kernels that ran
+    (platymatch_b200._lib.LAP_PATH).
     """
     torch = D._torch()
     c = np.asarray(cost_matrix)
@@ -55,5 +57,5 @@ def linear_sum_assignment(cost_matrix, maximize=False, return_stats=False, max_b
                                augmentations=int(st[2]), dijkstra_steps=int(st[3]), bids=int(st[5]),
                                refreshes=int(st[6]), retries=int(st[7]), parked=int(st[8]),
                                refresh_cycles=int(st[9]), auction_cycles=int(st[10]), bulk_bids=int(st[11]),
-                               sap_dense_relax=int(st[12]))
+                               sap_dense_relax=int(st[12]), path=int(st[13]))
     return rows, col

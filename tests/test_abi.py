@@ -64,8 +64,24 @@ def test_argument_validation_is_host_side():
     assert lib.pm_cloud_stats(None, 10, None, None) == -1
     assert b"null pointer" in lib.pm_last_error_string()
     assert lib.pm_lap_solve(None, 1, 4, 4, 4, 0, 0, None, None, None, None, 0, None) == -1
+    # more than 24 x 1024 columns: refused before any CUDA call (the pointers, 16-byte aligned and never read, stand
+    # in for device buffers)
+    p = ctypes.c_void_p(1 << 12)
+    for nr in (1, 24577):
+        assert lib.pm_lap_solve(p, 1, nr, 24577, 24580, 2048, 0, p, p, None, p, 1 << 40, None) == -5
+        assert b"nc = 24577 > 24576 columns not supported" in lib.pm_last_error_string()
     with pytest.raises(ValueError):
         _lib.check(-1, "x")
+
+
+def test_lap_path_bits_match_header():
+    """The Python names of the assignment's path bits are the header's PM_LAP_PATH_* values."""
+    from platymatch_b200 import _lib
+    text = open(os.path.join(ROOT, "include", "platymatch_b200.h")).read()
+    declared = {k: int(v) for k, v in re.findall(r"#define PM_LAP_PATH_([A-Z0-9_]+) (\d+)", text)}
+    assert declared == _lib.LAP_PATH
+    assert re.search(r"#define PM_LAP_STAT_PATH 13\b", text)
+    assert sorted(declared.values()) == [1 << k for k in range(len(declared))]
 
 
 def test_no_cpu_fallback_without_device():

@@ -88,8 +88,10 @@ def test_small_slack_exact(O, torch, slack):
 
 @pytest.mark.parametrize("env", [{"PM_LAP_BULK_PATIENCE": "0"}, {"PM_LAP_BULK_CTAS": "1"}, {"PM_LAP_BULK_CTAS": "400"},
                                  {"PM_LAP_BULK_STOP": "1"}, {"PM_LAP_STOP_LIVE": "0"}, {"PM_LAP_STOP_LIVE": "31"},
-                                 {"PM_LAP_EPS_SCALING": "0"}])
+                                 {"PM_LAP_EPS_SCALING": "0"}, {"PM_LAP_EPS_SCALING": "1"}])
 def test_auction_knobs_keep_exactness(O, torch, monkeypatch, env):
+    """Every tuning knob keeps the exact optimum.  PM_LAP_EPS_SCALING=1 squares the 1080 x 1200 problem as well
+    (120 dummy rows, far above the 2 % slack at which it is squared by default)."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     for n, dropout in ((1200, 0.1), (700, 0.0)):

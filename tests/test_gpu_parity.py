@@ -467,9 +467,10 @@ def test_supervised_8k_keypoints(O, torch):
 
 
 def test_registration_12k(O, torch):
-    """Beyond the 8k config: 10800 x 12000, sparse auction + sparse augmenting paths at a size where the tail
-    kernel's ring still fits in shared memory; the true hypothesis wins and the transform maps nuclei onto
-    their partners; the LAP cost does not exceed the ground-truth matching's on the same matrix."""
+    """Beyond the 8k config: 10800 x 12000, sparse auction (its ring still in shared memory) + DENSE augmenting paths
+    (the sparse ones would need 276 KB of shared memory at 12000 columns); the true hypothesis wins and the transform
+    maps nuclei onto their partners; the LAP cost does not exceed the ground-truth matching's on the same matrix.
+    Optimality against the oracle at this size: tests/test_gpu_lap_paths.py (P3)."""
     import platymatch_b200 as pm
     p = _pair(12000)
     res = pm.estimate_transform_unsupervised(p["moving"], p["fixed"], ransac_trials=2000, keep_cost=True, seed=1)
