@@ -78,6 +78,22 @@ int pm_label_centroids(const void *labels, int dtype, int nz, int ny, int nx, ui
                        int capacity, int32_t *ids, double *centroids, double *sizes, int32_t *n_out, void *workspace,
                        size_t workspace_bytes, void *stream);
 
+/* ---- resample a volume through an affine map (SURVEY §8f row 5) --------------------------------------
+ * The transformed-image export of EvaluateMetrics._export_transformed_image (_dock_widget.py:1095-1130): the
+ * moving image resampled into the fixed image's grid, so the two can be overlaid voxel by voxel.  Contract:
+ * scipy.ndimage.affine_transform(src, M[:3,:3], offset=M[:3,3], output_shape, order, mode='constant', cval)
+ * in voxel index space (the reference goes through SimpleITK; agreement with that is not verified).
+ *   src    [sz][sy][sx] int32 (PM_LABEL_I32), uint16 (PM_LABEL_U16) or float32 (PM_RESAMPLE_F32), device
+ *   M      16 float64, device: maps an output index (z, y, x, 1) to a source index; for a registration transform
+ *          T (moving zyx -> fixed zyx) this is inv(T).  c_h = ((z M[h][0] + y M[h][1]) + x M[h][2]) + M[h][3] in
+ *          float64 without FMA; an output voxel with any c_h NaN, < 0 or > n_h - 1 gets cval
+ *   order  0: src[floor(c + 0.5)];  1: trilinear in float64, neighbours past the last voxel clamped
+ *   dst    [dz][dy][dx], same dtype; float32 rounds to nearest, integers round half away from zero and saturate
+ * No workspace; src and dst must not overlap.  Offsets are 64-bit (volumes above 2^31 voxels are fine). */
+#define PM_RESAMPLE_F32 2
+int pm_resample_affine(const void *src, int dtype, int sz, int sy, int sx, const double *M, int order, double cval,
+                       void *dst, int dz, int dy, int dx, void *stream);
+
 /* ---- Euclidean distance matrix (SURVEY §8f row 3) ----------------------------------------------
  * scipy.spatial.distance.cdist as called by EvaluateMetrics._calculate_metrics (_dock_widget.py:1032,
  * 1038,1050): out[i * ldo + j] = ||a_i - b_j|| (float64 arithmetic, stored as the float32 costs the

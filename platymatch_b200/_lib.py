@@ -17,6 +17,7 @@ LAP_PATH = {"SQUARED": 1, "SPARSE_AUCTION": 2, "DENSE_AUCTION": 4, "SAP_SPARSE":
 CHI2_EPS = 2.0 ** -60
 CHI2_TILE = 128
 TRANSFORMS = {"Affine": 0, "Similar": 1}      # PM_TRANSFORM_* (the widget's strings, _dock_widget.py:627)
+VOLUME_DTYPES = {"int32": 0, "uint16": 1, "float32": 2}    # PM_LABEL_I32, PM_LABEL_U16, PM_RESAMPLE_F32
 
 _vp, _i, _d, _sz, _u64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_double, ctypes.c_size_t, ctypes.c_ulonglong
 
@@ -31,6 +32,7 @@ SIGNATURES = {
     "pm_label_max_id": (_i, [_vp, _i, _sz, _vp, _vp]),
     "pm_label_workspace_bytes": (_sz, [ctypes.c_uint32]),
     "pm_label_centroids": (_i, [_vp, _i, _i, _i, _i, ctypes.c_uint32, _d, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pm_resample_affine": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _d, _vp, _i, _i, _i, _vp]),
     "pm_cdist": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp]),
     "pm_cloud_stats": (_i, [_vp, _i, _vp, _vp]),
     "pm_mean_distance_workspace_bytes": (_sz, [_i]),

@@ -264,6 +264,34 @@ def label_centroids(labels, anisotropy=1.0, table_size=None, sync=True):
     return ids[:n], cen[:n], sizes[:n]
 
 
+def resample_affine(src, M, out_shape, order=0, cval=0.0, out=None):
+    """Volume src [sz, sy, sx] (CUDA int32, uint16 or float32 tensor) resampled into out_shape (dz, dy, dx), same dtype.
+    M: 4 x 4 float64 (CUDA tensor, or host array copied over) mapping an output voxel index (z, y, x, 1) to a source
+    index; order 0 (nearest) or 1 (trilinear); voxels that map outside the source get cval.  Equal to
+    scipy.ndimage.affine_transform(src, M[:3, :3], offset=M[:3, 3], output_shape, order, mode='constant', cval)
+    (pm_resample_affine).  out: a caller-owned contiguous tensor of that shape and dtype."""
+    torch = _torch()
+    name = str(src.dtype).replace("torch.", "")
+    if name not in _lib.VOLUME_DTYPES:
+        raise ValueError("volume must be int32, uint16 or float32, got %s" % src.dtype)
+    if not src.is_cuda or (out is not None and (not out.is_cuda or out.device != src.device)):
+        raise ValueError("src and out must be CUDA tensors on the same device")
+    if src.dim() != 3 or len(out_shape) != 3:
+        raise ValueError("expected a 3-D volume and a 3-D output shape")
+    if order not in (0, 1):
+        raise ValueError("order must be 0 or 1, got %r" % (order,))
+    src = src.contiguous()
+    m = torch.as_tensor(M, dtype=torch.float64, device=src.device).reshape(16).contiguous()
+    out_shape = tuple(int(s) for s in out_shape)
+    if out is None:
+        out = torch.empty(out_shape, dtype=src.dtype, device=src.device)
+    assert out.dtype == src.dtype and tuple(out.shape) == out_shape and out.is_contiguous()
+    sz, sy, sx = src.shape
+    check(load().pm_resample_affine(ptr(src), _lib.VOLUME_DTYPES[name], sz, sy, sx, ptr(m), int(order), float(cval),
+                                    ptr(out), *out_shape, stream_ptr()), "pm_resample_affine")
+    return out
+
+
 def cdist(a, b):
     """[n1,3], [n2,3] f64 -> [n1, ld] f32 Euclidean distances (ld = n2 rounded up to 4), as the LAP kernel wants them."""
     torch = _torch()
