@@ -182,6 +182,7 @@ int pm_chi2_cost(const float *a_t, int lda, const uint32_t *a_mask, int n1, cons
 #define PM_LAP_STAT_BULK_BIDS 11      /* sparse auction: bids made by the multi-SM bulk kernel */
 #define PM_LAP_STAT_SAP_DENSE_RELAX 12 /* sparse augmenting paths: tree rows that had to be relaxed densely */
 #define PM_LAP_STAT_PATH 13           /* kernels this solve ran: PM_LAP_PATH_* bits */
+#define PM_LAP_STAT_SAP_CYCLES 14     /* sparse augmenting paths: SM cycles of pm_lap_sap_sparse_kernel, entry to exit */
 /* path bits: squared with dummy rows; the auction that ran (neither bit: max_bid_rounds = 0, augmenting paths only);
  * exactly one finishing kernel; the sparse auction's ring of displaced rows in shared memory (else global memory) */
 #define PM_LAP_PATH_SQUARED 1

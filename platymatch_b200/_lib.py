@@ -11,6 +11,9 @@ LIB_PATH = os.path.join(_HERE, "libplatymatch_b200.so")
 
 NBINS = 360
 LAP_STATS = 16
+# PM_LAP_STAT_* slots of the assignment's statistics that Python code reads by name
+LAP_STAT = {"DIJKSTRA_STEPS": 3, "BIDS": 5, "REFRESHES": 6, "REFRESH_CYCLES": 9, "AUCTION_CYCLES": 10,
+            "SAP_DENSE_RELAX": 12, "PATH": 13, "SAP_CYCLES": 14}
 # PM_LAP_PATH_* bits of the assignment's `path` statistic (PM_LAP_STAT_PATH): which kernels a solve ran
 LAP_PATH = {"SQUARED": 1, "SPARSE_AUCTION": 2, "DENSE_AUCTION": 4, "SAP_SPARSE": 8, "SAP_DENSE8": 16,
             "SAP_DENSE16": 32, "SAP_DENSE24": 64, "RING_SMEM": 128}

@@ -1254,35 +1254,49 @@ __global__ void __launch_bounds__(PM_LAP_MAX_THREADS, 1) pm_lap_sap_kernel(PmLap
 // is <= the smallest bound over the tree; otherwise the row holding that bound is relaxed densely
 // (exactly the dense algorithm's step) and its bound removed.  Same result as the dense search.
 //
-// dynamic shared memory: v f64[ncp] | d f64[ncp] | pred u16[ncp] | r4c u16[ncp] | front u16[ncp] | scanned u8[ncp]
-#define PM_SS_THREADS 1024     // the reached frontier grows to most of the columns within ~60 steps: the scan wants every thread
+// The steps are serial, so ONE warp runs them, without block barriers.  The columns are split into
+// segments of PM_SS_SEG; shared memory keeps per segment the smallest pm_ordkey(d) over its unscanned
+// columns.  A step relaxes the new tree row's list (4 entries per lane; an improved d lowers its segment's
+// key with a shared atomicMin), takes the arg-min over the segment keys and scans only the winning
+// segment, for its lowest column at that distance, whose key it then recomputes without that column.
+// Segments are contiguous and ties go to the lower segment, so columns are finalised in the order of a
+// full scan: smallest distance first, the lower column index on a tie.  (d is never -0: costs enter as
+// dist + c with dist starting at +0, so key order is value order.)  The other warps wait on a named
+// barrier and join only for the dense relaxation of a tree row; the per-augmentation reset, the dual
+// update and the augmentation use the whole CTA.
+//
+// dynamic shared memory: v f64[ncp] | d f64[ncp] | pred u16[ncp] | r4c u16[ncp] | scanned u8[ncp]
+#define PM_SS_THREADS 1024     // the dense relaxation of a tree row and the per-augmentation work want every thread
+#define PM_SS_SEG 256          // columns per segment: one warp, 8 per lane
+#define PM_SS_MAX_SEGS 64      // two per lane of the stepping warp
+// Largest padded column count this kernel is selected for.  It is where the kernel's former layout (23 B of shared
+// memory per column) stopped fitting the 227 KB of a B200; the dense kernels are measured and tested from there on.
+#define PM_SS_MAX_COLS 10016
+#define PM_SS_CMD_DENSE 1      // s_cmd: relax tree row s_il densely
+#define PM_SS_CMD_DONE 2       // s_cmd: the search of this augmentation is over (s_sink, s_status, s_min)
 
-// warp arg-min over (value, tie) in lexicographic order with three REDUX instead of 15 shuffles
-__device__ __forceinline__ void pm_ss_argmin_warp(double &val, int &tie) {
-    const unsigned long long k = pm_ordkey(val);
-    const unsigned long long kb = pm_warp_min_u64(k);
-    tie = (int)__reduce_min_sync(0xffffffffu, k == kb ? (unsigned)tie : 0xffffffffu);
-    val = pm_ordval(kb);
-}
+// barrier 1 over the whole CTA: the stepping warp hands work to the waiting warps without __syncthreads
+__device__ __forceinline__ void pm_ss_bar() { asm volatile("bar.sync 1, %0;" ::"n"(PM_SS_THREADS) : "memory"); }
 
 __global__ void __launch_bounds__(PM_SS_THREADS, 1) pm_lap_sap_sparse_kernel(PmLapBatch B) {
     extern __shared__ __align__(16) unsigned char pm_ss_smem[];
+    const long long t_entry = clock64();               // (thread 0's reading is reported as PM_LAP_STAT_SAP_CYCLES)
     const PmLapView V = pm_lap_view(B, blockIdx.x);
     const int nc = B.nc, nr = B.nr, ncp = B.ncp, ldc = B.ldc;
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int nseg = (ncp + PM_SS_SEG - 1) / PM_SS_SEG;
+    const unsigned long long key_inf = pm_ordkey(INFINITY);
     double *v = reinterpret_cast<double *>(pm_ss_smem);
     double *d = v + ncp;
     unsigned short *pred = reinterpret_cast<unsigned short *>(d + ncp);
     unsigned short *r4c = pred + ncp;
-    unsigned short *front = r4c + ncp;             // columns reached so far in this search (finite distance)
-    unsigned char *scanned = reinterpret_cast<unsigned char *>(front + ncp);
-    __shared__ int s_nfront;
-    __shared__ double s_val[2][32];
-    __shared__ int s_tie[2][32];
+    unsigned char *scanned = reinterpret_cast<unsigned char *>(r4c + ncp);
+    __shared__ unsigned long long s_seg[PM_SS_MAX_SEGS];   // per segment: min pm_ordkey(d) over its unscanned columns
+    __shared__ double s_sum[32];
     __shared__ int s_scan[33];
     __shared__ int s_nfree;
-    __shared__ double s_lam;
-    __shared__ int s_lam_idx;
+    __shared__ int s_cmd, s_il, s_sink, s_status;
+    __shared__ double s_dl, s_min;
     int32_t *tree_row = V.bid_col;                 // [nr] scratch of the dense auction, free here
     double *tree_dist = V.bid_gamma;               // [nr]
     double *tree_bound = reinterpret_cast<double *>(V.colbest);   // [nc] >= [nr]
@@ -1314,102 +1328,157 @@ __global__ void __launch_bounds__(PM_SS_THREADS, 1) pm_lap_sap_sparse_kernel(PmL
         __syncthreads();
     }
     const int nfree = s_nfree;
-    long long steps = 0, dense_relax = 0;
-    int status = 0, parity = 0;
+    long long steps = 0, dense_relax = 0;          // (counted by the stepping warp)
+    int status = 0;
+
+    // every warp: relax tree row s_il (distance s_dl) densely over the segments it owns, then recompute their keys
+    auto dense_relax_row = [&]() {
+        const int il = s_il;
+        const double dl = s_dl, uil = __ldcg(V.u + il);
+        const float *ci = pm_lap_row(V.cost, B, il);
+        for (int sg = warp; sg < nseg; sg += PM_SS_THREADS / 32) {
+            const int base = sg * PM_SS_SEG + lane;
+            float c[PM_SS_SEG / 32];
+#pragma unroll
+            for (int q = 0; q < PM_SS_SEG / 32; ++q) c[q] = (base + 32 * q < nc) ? ci[base + 32 * q] : 0.f;
+            unsigned long long m = key_inf;
+#pragma unroll
+            for (int q = 0; q < PM_SS_SEG / 32; ++q) {
+                const int j = base + 32 * q;
+                if (j < nc && !scanned[j]) {
+                    const double r = ((dl + (double)c[q]) - uil) - v[j];
+                    double dj = d[j];
+                    if (r < dj) { dj = r; d[j] = r; pred[j] = (unsigned short)il; }
+                    const unsigned long long k = pm_ordkey(dj);
+                    if (k < m) m = k;
+                }
+            }
+            m = pm_warp_min_u64(m);
+            if (lane == 0) s_seg[sg] = m;
+        }
+    };
 
     for (int f = 0; f < nfree && status == 0; ++f) {
         const int cur = flist[f];
         for (int j = t; j < ncp; j += PM_SS_THREADS) { d[j] = INFINITY; scanned[j] = 0; }
-        if (t == 0) { s_lam = INFINITY; s_lam_idx = -1; s_nfront = 0; }
+        if (t < PM_SS_MAX_SEGS) s_seg[t] = key_inf;
         __syncthreads();
-        int i = cur, sink = -1, nt = 0, jlast = -1;      // jlast: column finalised in the previous step
-        double dist = 0.0, min_val = 0.0;
-        while (sink < 0 && status == 0) {
-            // ---- add row i (distance dist) to the tree: relax its list edges, record its bound
-            const double ui = __ldcg(V.u + i);
-            if (t < PM_LS_K) {
-                const int j = __ldcg(V.lcol + (size_t)i * PM_LS_K + t);          // both list loads in flight together
-                const float cij = __ldcg(V.lcost + (size_t)i * PM_LS_K + t);
-                if (j >= 0 && j != jlast && !scanned[j]) {     // (its scanned flag may not be visible yet)
-                    const double r = ((dist + (double)cij) - ui) - v[j];
-                    const double old = d[j];
-                    if (r < old) {
-                        if (!(old < INFINITY)) front[atomicAdd(&s_nfront, 1)] = (unsigned short)j;   // first time reached
-                        d[j] = r; pred[j] = (unsigned short)i;
-                    }
+        if (warp == 0) {
+            int i = cur, sink = -1, nt = 0, lam_idx = -1;
+            double dist = 0.0, min_val = 0.0, lam = INFINITY;   // lam: smallest bound over the tree (row lam_idx)
+            // the list of the row that joins the tree next: loaded as soon as the row is known (one L2 round trip,
+            // every load in flight together), so that the bookkeeping of the step that found it hides part of the trip
+            double ui, taui;
+            int lj[PM_LS_K / 32];
+            float lc[PM_LS_K / 32];
+            auto load_row = [&](int row) {
+                ui = __ldcg(V.u + row); taui = __ldcg(V.tau + row);
+#pragma unroll
+                for (int q = 0; q < PM_LS_K / 32; ++q) {
+                    lj[q] = __ldcg(V.lcol + (size_t)row * PM_LS_K + lane + 32 * q);
+                    lc[q] = __ldcg(V.lcost + (size_t)row * PM_LS_K + lane + 32 * q);
                 }
-            } else if (t == PM_LS_K) {
-                const double bound = (dist + __ldcg(V.tau + i)) - ui;
-                tree_row[nt] = i; tree_dist[nt] = dist; tree_bound[nt] = bound;
-                if (bound < s_lam) { s_lam = bound; s_lam_idx = nt; }
-            }
-            ++nt;
-            __syncthreads();
-            while (true) {
-                // ---- closest unscanned column (ties: the lower index)
-                double best = INFINITY;
-                int best_tie = INT_MAX;
-                const int nfront = s_nfront;
-                for (int q = t; q < nfront; q += PM_SS_THREADS) {
-                    const int j = front[q];
-                    if (!scanned[j]) {
-                        const double dj = d[j];
-                        if (dj < best || (dj == best && j < best_tie)) { best = dj; best_tie = j; }
-                    }
+            };
+            load_row(i);
+            while (sink < 0 && status == 0) {
+                // ---- add row i (distance dist) to the tree: relax its list edges, record its bound
+                unsigned char sc[PM_LS_K / 32];
+                double vj[PM_LS_K / 32], dj[PM_LS_K / 32];
+#pragma unroll
+                for (int q = 0; q < PM_LS_K / 32; ++q) {
+                    const int j = lj[q] < 0 ? 0 : lj[q];
+                    sc[q] = scanned[j]; vj[q] = v[j]; dj[q] = d[j];
                 }
-                pm_ss_argmin_warp(best, best_tie);
-                if (lane == 0) { s_val[parity][warp] = best; s_tie[parity][warp] = best_tie; }
-                __syncthreads();
-                best = (lane < PM_SS_THREADS / 32) ? s_val[parity][lane] : INFINITY;
-                best_tie = (lane < PM_SS_THREADS / 32) ? s_tie[parity][lane] : INT_MAX;
-                pm_ss_argmin_warp(best, best_tie);
-                parity ^= 1;
-                const double lam = s_lam;
-                const int lam_idx = s_lam_idx;
-                if (best <= lam) {
-                    if (!(best < INFINITY)) { status = PM_ERR_INFEASIBLE; break; }
-                    ++steps;
-                    min_val = best;
-                    const int jm = best_tie;
-                    if (t == 0) scanned[jm] = 1;                // visible to everybody after the next barrier
-                    jlast = jm;
-                    if (r4c[jm] == PM_LS_NONE) sink = jm;
-                    else { i = r4c[jm]; dist = best; }
-                    break;
-                }
-                // ---- an edge outside the list of tree row `il` could be shorter: relax that row densely
-                __syncthreads();                               // everybody has read s_lam
-                const int il = tree_row[lam_idx];
-                const double dl = tree_dist[lam_idx], uil = __ldcg(V.u + il);
-                const float *ci = pm_lap_row(V.cost, B, il);
-                for (int j = t; j < nc; j += PM_SS_THREADS) {
-                    if (!scanned[j]) {
-                        const double r = ((dl + (double)ci[j]) - uil) - v[j];
-                        const double old = d[j];
-                        if (r < old) {
-                            if (!(old < INFINITY)) front[atomicAdd(&s_nfront, 1)] = (unsigned short)j;
-                            d[j] = r; pred[j] = (unsigned short)il;
+#pragma unroll
+                for (int q = 0; q < PM_LS_K / 32; ++q) {
+                    const int j = lj[q];
+                    if (j >= 0 && !sc[q]) {
+                        const double r = ((dist + (double)lc[q]) - ui) - vj[q];
+                        if (r < dj[q]) {
+                            d[j] = r; pred[j] = (unsigned short)i;
+                            atomicMin(&s_seg[j / PM_SS_SEG], pm_ordkey(r));
                         }
                     }
                 }
-                ++dense_relax;
-                if (t == 0) tree_bound[lam_idx] = INFINITY;
-                __syncthreads();
-                if (warp == 0) {                               // smallest remaining bound over the tree
-                    double lb = INFINITY;
+                const double bound = (dist + taui) - ui;
+                if (lane == 0) { tree_row[nt] = i; tree_dist[nt] = dist; tree_bound[nt] = bound; }
+                if (bound < lam) { lam = bound; lam_idx = nt; }
+                ++nt;
+                __syncwarp();
+                while (true) {
+                    // ---- closest unscanned column: the lowest segment holding the smallest key, then its lowest column
+                    const unsigned long long k0 = s_seg[lane], k1 = s_seg[lane + 32];
+                    const unsigned long long key = k1 < k0 ? k1 : k0;
+                    const int seg = k1 < k0 ? lane + 32 : lane;
+                    const unsigned long long kb = pm_warp_min_u64(key);
+                    const double best = pm_ordval(kb);
+                    if (best <= lam) {
+                        if (!(best < INFINITY)) { status = PM_ERR_INFEASIBLE; break; }
+                        const int sb = (int)__reduce_min_sync(0xffffffffu, key == kb ? (unsigned)seg : 0xffffffffu);
+                        const int base = sb * PM_SS_SEG + lane;
+                        unsigned char s8[PM_SS_SEG / 32];
+                        double dd[PM_SS_SEG / 32];
+#pragma unroll
+                        for (int q = 0; q < PM_SS_SEG / 32; ++q) {
+                            const int j = base + 32 * q < nc ? base + 32 * q : nc - 1;
+                            s8[q] = scanned[j]; dd[q] = d[j];
+                        }
+                        unsigned long long ck[PM_SS_SEG / 32];
+                        unsigned jl = 0xffffffffu;
+#pragma unroll
+                        for (int q = 0; q < PM_SS_SEG / 32; ++q) {
+                            ck[q] = (base + 32 * q < nc && !s8[q]) ? pm_ordkey(dd[q]) : key_inf;
+                            if (ck[q] == kb && jl == 0xffffffffu) jl = (unsigned)(base + 32 * q);
+                        }
+                        const int jm = (int)__reduce_min_sync(0xffffffffu, jl);
+                        const int r = r4c[jm];
+                        if (r == PM_LS_NONE) sink = jm;
+                        else { i = r; dist = best; load_row(i); }
+                        unsigned long long rest = key_inf;     // the segment's key without jm
+#pragma unroll
+                        for (int q = 0; q < PM_SS_SEG / 32; ++q)
+                            if (base + 32 * q != jm && ck[q] < rest) rest = ck[q];
+                        rest = pm_warp_min_u64(rest);
+                        if (lane == 0) s_seg[sb] = rest;
+                        if (lane == (jm & 31)) scanned[jm] = 1;
+                        ++steps;
+                        min_val = best;
+                        __syncwarp();
+                        break;
+                    }
+                    // ---- an edge outside the list of tree row `lam_idx` could be shorter: relax that row densely
+                    if (lane == 0) {
+                        s_cmd = PM_SS_CMD_DENSE; s_il = tree_row[lam_idx]; s_dl = tree_dist[lam_idx];
+                        tree_bound[lam_idx] = INFINITY;
+                    }
+                    pm_ss_bar();
+                    dense_relax_row();
+                    pm_ss_bar();                                 // every segment key is exact again
+                    ++dense_relax;
+                    lam = INFINITY;                              // smallest remaining bound over the tree
                     int li = INT_MAX;
                     for (int k = lane; k < nt; k += 32) {
                         const double bnd = tree_bound[k];
-                        if (bnd < lb || (bnd == lb && k < li)) { lb = bnd; li = k; }
+                        if (bnd < lam || (bnd == lam && k < li)) { lam = bnd; li = k; }
                     }
-                    pm_argmin_warp(lb, li);
-                    if (lane == 0) { s_lam = lb; s_lam_idx = (lb < INFINITY) ? li : -1; }
+                    pm_argmin_warp(lam, li);
+                    lam_idx = (lam < INFINITY) ? li : -1;
                 }
-                __syncthreads();
+            }
+            if (lane == 0) { s_cmd = PM_SS_CMD_DONE; s_sink = sink; s_status = status; s_min = min_val; }
+            pm_ss_bar();
+        } else {
+            while (true) {
+                pm_ss_bar();
+                if (s_cmd != PM_SS_CMD_DENSE) break;
+                dense_relax_row();
+                pm_ss_bar();
             }
         }
+        const int sink = s_sink;
+        const double min_val = s_min;
+        status = s_status;
         if (status) break;
-        __syncthreads();
         // dual update (Crouse: u[cur] += min; scanned rows / columns shift by min - d); prices only fall
         for (int j = t; j < nc; j += PM_SS_THREADS) {
             if (scanned[j]) {
@@ -1444,7 +1513,7 @@ __global__ void __launch_bounds__(PM_SS_THREADS, 1) pm_lap_sap_sparse_kernel(PmL
         V.col4row_out[r] = c;
         if (c >= 0) tot += (double)V.cost[(size_t)r * ldc + c];
     }
-    tot = pm_block_sum(tot, &s_val[0][0]);
+    tot = pm_block_sum(tot, s_sum);
     if (t == 0) {
         V.total[0] = status ? nan("") : tot;
         V.counters[4] = status;
@@ -1456,6 +1525,7 @@ __global__ void __launch_bounds__(PM_SS_THREADS, 1) pm_lap_sap_sparse_kernel(PmL
             V.stats[PM_LAP_STAT_STATUS] = status;
             V.stats[PM_LAP_STAT_SAP_DENSE_RELAX] = dense_relax;
             V.stats[PM_LAP_STAT_PATH] = B.path;
+            V.stats[PM_LAP_STAT_SAP_CYCLES] = clock64() - t_entry;
         }
     }
 }
@@ -1664,8 +1734,9 @@ extern "C" int pm_lap_solve(const float *cost, int batch, int nr, int nc, int ld
         PM_LAUNCH_CHECK();
     }
     int rc;
-    const size_t ss_smem = (size_t)B.ncp * (8 + 8 + 2 + 2 + 2 + 1);
-    if (max_bid_rounds > 0 && algorithm == PM_LAP_ALGO_SPARSE_AUCTION && ss_smem + 2048 <= (size_t)smem_optin) {
+    const size_t ss_smem = (size_t)B.ncp * (8 + 8 + 2 + 2 + 1);
+    if (max_bid_rounds > 0 && algorithm == PM_LAP_ALGO_SPARSE_AUCTION && B.ncp <= PM_SS_MAX_COLS &&
+        ss_smem + 2048 <= (size_t)smem_optin) {
         if (int rc = pm_lap_raise_smem_limit(pm_lap_sap_sparse_kernel, smem_optin, dev)) return rc;
         B.path |= PM_LAP_PATH_SAP_SPARSE;
         pm_lap_sap_sparse_kernel<<<batch, PM_SS_THREADS, ss_smem, s>>>(B);

@@ -57,5 +57,5 @@ def linear_sum_assignment(cost_matrix, maximize=False, return_stats=False, max_b
                                augmentations=int(st[2]), dijkstra_steps=int(st[3]), bids=int(st[5]),
                                refreshes=int(st[6]), retries=int(st[7]), parked=int(st[8]),
                                refresh_cycles=int(st[9]), auction_cycles=int(st[10]), bulk_bids=int(st[11]),
-                               sap_dense_relax=int(st[12]), path=int(st[13]))
+                               sap_dense_relax=int(st[12]), path=int(st[13]), sap_cycles=int(st[14]))
     return rows, col
