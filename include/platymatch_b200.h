@@ -94,6 +94,42 @@ int pm_label_centroids(const void *labels, int dtype, int nz, int ny, int nx, ui
 int pm_resample_affine(const void *src, int dtype, int sz, int sy, int sx, const double *M, int order, double cval,
                        void *dst, int dz, int dy, int dx, void *stream);
 
+/* ---- nuclei detection: scale-space LoG (SURVEY §2 row 10) --------------------------------------------------
+ * DetectNuclei / find_spheres (platymatch/detect_nuclei/ss_log.py:25-87).  The contract is this project's own
+ * (DESIGN §8 row 6; the reference's parameters are not available and agreement with it is unverified):
+ * L_k = float32(sigma_k^2) * gaussian_laplace(img, (sigma_k / a, sigma_k, sigma_k)) as 8 separable passes, (value,
+ * index) minima over 3x3x3x3 above 0.2 x Otsu, greedy sphere-overlap suppression.  Offsets are 64-bit.
+ *
+ * pm_detect_pass: one 1-D correlation of src [nz][ny][nx] float32 along `axis` (0 z, 1 y, 2 x) with the symmetric
+ *   float64 weights w[0..lw] (centre, then offsets 1..lw; device), mode 'reflect', float64 accumulation in scipy's
+ *   order (centre, then tap pairs outermost first), float32 result.  t0, t1 non-NULL: dst = scale * ((t0 + t1) + v)
+ *   in float32 (the Laplacian's sum and scale-normalisation).  lw <= 384; src, t0, t1 must not overlap dst. */
+int pm_detect_pass(const float *src, int nz, int ny, int nx, int axis, const double *weights, int lw, const float *t0,
+                   const float *t1, float scale, float *dst, void *stream);
+/* pm_detect_otsu: out[0] = skimage's threshold_otsu(img, nbins=256) (np.histogram binning of float32 data with float32
+ *   edges, float64 statistics, first maximum; a constant image gives its value), out[1] = factor * out[0]; device. */
+size_t pm_detect_otsu_workspace_bytes(void);
+int pm_detect_otsu(const float *img, size_t n, double factor, double *out, void *workspace, size_t workspace_bytes,
+                   void *stream);
+/* pm_detect_minima: scale k's candidates.  l_prev / l_next are L_{k-1} / L_{k+1} (NULL = absent).  A voxel whose
+ *   (L, linear index in (k, z, y, x) order) is strictly smaller than that of every present neighbour of its 3x3x3x3
+ *   neighbourhood, and with -(double)L > threshold[1], is appended: keys[pos] = linear index, values[pos] = L, pos from
+ *   *count (uint64, device, accumulated across calls; the caller zeroes it).  *count > capacity: the candidates past
+ *   capacity were not stored; retry with more.  At most one candidate lies in any 2x2x2x2 block. */
+int pm_detect_minima(const float *l_prev, const float *l_cur, const float *l_next, int nz, int ny, int nx, int k,
+                     const double *threshold, long long capacity, long long *keys, float *values,
+                     unsigned long long *count, void *stream);
+/* pm_detect_suppress: keys [capacity] sorted by priority, the first min(*count, capacity) are the candidates.  Each is a
+ *   sphere at (z * anisotropy, y, x) of radius radii[k] (device, every radius <= max_radius).  In priority order a
+ *   candidate is kept unless its lens volume with an already kept sphere is greater than overlap x the smaller
+ *   sphere's volume (float64, no FMA; same formula as ss_log.sphere_intersection).  state[i] = 1 kept, 2 dropped.
+ *   workspace: pm_detect_suppress_workspace_bytes(capacity, nz, ny, nx, max_radius, anisotropy). */
+size_t pm_detect_suppress_workspace_bytes(long long capacity, int nz, int ny, int nx, double max_radius,
+                                          double anisotropy);
+int pm_detect_suppress(const long long *keys, const unsigned long long *count, long long capacity, int nz, int ny,
+                       int nx, const double *radii, double max_radius, double anisotropy, double overlap,
+                       unsigned char *state, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- Euclidean distance matrix (SURVEY §8f row 3) ----------------------------------------------
  * scipy.spatial.distance.cdist as called by EvaluateMetrics._calculate_metrics (_dock_widget.py:1032,
  * 1038,1050): out[i * ldo + j] = ||a_i - b_j|| (float64 arithmetic, stored as the float32 costs the

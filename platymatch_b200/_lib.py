@@ -36,6 +36,12 @@ SIGNATURES = {
     "pm_label_workspace_bytes": (_sz, [ctypes.c_uint32]),
     "pm_label_centroids": (_i, [_vp, _i, _i, _i, _i, ctypes.c_uint32, _d, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pm_resample_affine": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _d, _vp, _i, _i, _i, _vp]),
+    "pm_detect_pass": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, ctypes.c_float, _vp, _vp]),
+    "pm_detect_otsu_workspace_bytes": (_sz, []),
+    "pm_detect_otsu": (_i, [_vp, _sz, _d, _vp, _vp, _sz, _vp]),
+    "pm_detect_minima": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, ctypes.c_longlong, _vp, _vp, _vp, _vp]),
+    "pm_detect_suppress_workspace_bytes": (_sz, [ctypes.c_longlong, _i, _i, _i, _d, _d]),
+    "pm_detect_suppress": (_i, [_vp, _vp, ctypes.c_longlong, _i, _i, _i, _vp, _d, _d, _d, _vp, _vp, _sz, _vp]),
     "pm_cdist": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp]),
     "pm_cloud_stats": (_i, [_vp, _i, _vp, _vp]),
     "pm_mean_distance_workspace_bytes": (_sz, [_i]),

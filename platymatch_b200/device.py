@@ -371,3 +371,52 @@ class PeerWindow:
         if self.ptr:
             load().pm_peer_free(ctypes.c_void_p(self.ptr))
             self.ptr = None
+
+
+def detect_pass(src, axis, weights, out=None, t0=None, t1=None, scale=1.0):
+    """One separable 1-D correlation of a float32 CUDA volume along `axis` (pm_detect_pass): weights = the symmetric
+    float64 half-kernel w[0..lw] (centre first, CUDA tensor), mode 'reflect', float32 result.  t0 / t1 given:
+    out = scale * ((t0 + t1) + pass) in float32."""
+    torch = _torch()
+    assert src.dtype == torch.float32 and src.dim() == 3 and src.is_cuda and src.is_contiguous()
+    assert weights.dtype == torch.float64 and weights.is_cuda and weights.is_contiguous()
+    if out is None:
+        out = torch.empty_like(src)
+    nz, ny, nx = src.shape
+    check(load().pm_detect_pass(ptr(src), nz, ny, nx, int(axis), ptr(weights), weights.numel() - 1, ptr(t0), ptr(t1),
+                                float(scale), ptr(out), stream_ptr()), "pm_detect_pass")
+    return out
+
+
+def detect_otsu(img, factor=1.0):
+    """[2] float64 device tensor: (threshold_otsu(img, 256), factor * threshold) of a float32 CUDA tensor."""
+    torch = _torch()
+    assert img.dtype == torch.float32 and img.is_cuda and img.is_contiguous()
+    out = torch.empty(2, dtype=torch.float64, device=img.device)
+    nbytes = load().pm_detect_otsu_workspace_bytes()
+    ws = torch.empty(nbytes // 8 + 1, dtype=torch.int64, device=img.device)
+    check(load().pm_detect_otsu(ptr(img), img.numel(), float(factor), ptr(out), ptr(ws), nbytes, stream_ptr()),
+          "pm_detect_otsu")
+    return out
+
+
+def detect_minima(l_prev, l_cur, l_next, k, threshold, keys, values, count):
+    """Append scale k's candidates (pm_detect_minima) to keys [cap] int64 / values [cap] float32; count [1] int64."""
+    nz, ny, nx = l_cur.shape
+    check(load().pm_detect_minima(ptr(l_prev), ptr(l_cur), ptr(l_next), nz, ny, nx, int(k), ptr(threshold),
+                                  keys.numel(), ptr(keys), ptr(values), ptr(count), stream_ptr()), "pm_detect_minima")
+
+
+def detect_suppress(keys, count, shape, radii, max_radius, anisotropy, overlap):
+    """Greedy suppression of the priority-sorted candidates keys [cap] (the first min(count, cap)); radii: CUDA float64
+    per scale.  -> state [cap] uint8 (1 kept, 2 dropped; entries past the count are undefined)."""
+    torch = _torch()
+    cap = keys.numel()
+    nz, ny, nx = shape
+    state = torch.empty(cap, dtype=torch.uint8, device=keys.device)
+    nbytes = load().pm_detect_suppress_workspace_bytes(cap, nz, ny, nx, float(max_radius), float(anisotropy))
+    ws = torch.empty(nbytes // 8 + 1, dtype=torch.int64, device=keys.device)
+    check(load().pm_detect_suppress(ptr(keys), ptr(count), cap, nz, ny, nx, ptr(radii), float(max_radius),
+                                    float(anisotropy), float(overlap), ptr(state), ptr(ws), nbytes, stream_ptr()),
+          "pm_detect_suppress")
+    return state

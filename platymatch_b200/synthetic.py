@@ -7,7 +7,8 @@ the registration path.  Clouds are modelled on the reference's test assets
 """
 import numpy as np
 
-__all__ = ["make_fixed_cloud", "random_affine", "make_pair", "make_keypoints", "make_specimens"]
+__all__ = ["make_fixed_cloud", "random_affine", "make_pair", "make_keypoints", "make_specimens", "make_label_volume",
+           "make_nuclei_image"]
 
 
 def make_fixed_cloud(n, rng, filled=False):
@@ -114,3 +115,23 @@ def make_label_volume(shape=(64, 96, 128), n_nuclei=60, radius=(3.0, 6.0), seed=
         sub = ((zz[z0:z1] - c[0]) ** 2 + (yy[:, y0:y1] - c[1]) ** 2 + (xx[:, :, x0:x1] - c[2]) ** 2) <= r * r
         vol[z0:z1, y0:y1, x0:x1][sub] = ids[k]
     return vol.astype(dtype)
+
+
+def make_nuclei_image(shape, centers, radius, contrast=100.0, background=10.0, noise=2.0, seed=0):
+    """float32 intensity volume of nuclei-stained nuclei: background + contrast x a Gaussian blob of sigma = radius / 2
+    at each (z, y, x) centre (radius: scalar or one per centre, voxels), plus Gaussian noise of std `noise`."""
+    rng = np.random.default_rng(seed)
+    centers = np.asarray(centers, dtype=np.float64).reshape(-1, 3)
+    rad = np.broadcast_to(np.asarray(radius, dtype=np.float64), (len(centers),))
+    vol = np.full(shape, float(background), dtype=np.float64)
+    for c, r in zip(centers, rad):
+        s = r / 2.0
+        lo = [max(int(np.floor(c[h] - 4 * s)), 0) for h in range(3)]
+        hi = [min(int(np.ceil(c[h] + 4 * s)) + 1, shape[h]) for h in range(3)]
+        if any(a >= b for a, b in zip(lo, hi)):
+            continue
+        g = [np.exp(-0.5 * ((np.arange(lo[h], hi[h]) - c[h]) / s) ** 2) for h in range(3)]
+        vol[lo[0]:hi[0], lo[1]:hi[1], lo[2]:hi[2]] += contrast * g[0][:, None, None] * g[1][None, :, None] * g[2]
+    if noise:
+        vol += rng.normal(0.0, noise, size=shape)
+    return vol.astype(np.float32)
