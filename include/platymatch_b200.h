@@ -78,6 +78,24 @@ int pm_label_centroids(const void *labels, int dtype, int nz, int ny, int nx, ui
                        int capacity, int32_t *ids, double *centroids, double *sizes, int32_t *n_out, void *workspace,
                        size_t workspace_bytes, void *stream);
 
+/* ---- two label volumes -> contingency table (DESIGN §8 row 7) ------------------------------------------------
+ * What a segmentation is scored with when there are no keypoints: for volumes A, B of one shape, every pair of ids
+ * (a, b) != (0, 0) that meet at some voxel and its voxel count (np.unique of the pair keys a << 32 | b with the
+ * (0, 0) entry removed).  Ids <= 0 count as background (0).  Instance sizes are the table's row and column sums,
+ * IoU(a, b) = n / (|A_a| + |B_b| - n).  One streaming pass over both volumes (HBM-bound) into an open-addressing hash
+ * table of `capacity` slots in the workspace, then a compaction.  Offsets and counts are 64-bit.
+ *   labels_a, labels_b  [nz][ny][nx] int32 (PM_LABEL_I32) or uint16 (PM_LABEL_U16) each, device
+ *   capacity   table slots, a power of two; a pair that finds no slot within 128 probes is not stored (keep the
+ *              table at most half full: pm_label_max_id of both volumes bounds the number of pairs in practice)
+ *   keys [capacity] uint64 out: a << 32 | b of the first n_out[0] entries, any order;  counts [capacity] uint64 out
+ *   n_out [2] uint64 out: pairs written, voxels whose pair was NOT stored (non-zero = overflow: rerun with a larger
+ *              capacity; the pairs written are then incomplete)
+ * Every pointer must be 16-byte aligned.  workspace: pm_label_overlap_workspace_bytes(capacity). */
+size_t pm_label_overlap_workspace_bytes(uint64_t capacity);
+int pm_label_overlap(const void *labels_a, int dtype_a, const void *labels_b, int dtype_b, int nz, int ny, int nx,
+                     uint64_t capacity, uint64_t *keys, uint64_t *counts, uint64_t *n_out, void *workspace,
+                     size_t workspace_bytes, void *stream);
+
 /* ---- resample a volume through an affine map (SURVEY §8f row 5) --------------------------------------
  * The transformed-image export of EvaluateMetrics._export_transformed_image (_dock_widget.py:1095-1130): the
  * moving image resampled into the fixed image's grid, so the two can be overlaid voxel by voxel.  Contract:

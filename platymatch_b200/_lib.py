@@ -35,6 +35,8 @@ SIGNATURES = {
     "pm_label_max_id": (_i, [_vp, _i, _sz, _vp, _vp]),
     "pm_label_workspace_bytes": (_sz, [ctypes.c_uint32]),
     "pm_label_centroids": (_i, [_vp, _i, _i, _i, _i, ctypes.c_uint32, _d, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pm_label_overlap_workspace_bytes": (_sz, [_u64]),
+    "pm_label_overlap": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _u64, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pm_resample_affine": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _d, _vp, _i, _i, _i, _vp]),
     "pm_detect_pass": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, ctypes.c_float, _vp, _vp]),
     "pm_detect_otsu_workspace_bytes": (_sz, []),

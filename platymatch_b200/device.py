@@ -264,6 +264,47 @@ def label_centroids(labels, anisotropy=1.0, table_size=None, sync=True):
     return ids[:n], cen[:n], sizes[:n]
 
 
+def _label_dtype_code(t):
+    torch = _torch()
+    if t.dtype == torch.int32:
+        return 0
+    if t.dtype == torch.uint16:
+        return 1
+    raise ValueError("label volume must be int32 or uint16, got %s" % t.dtype)
+
+
+def label_max_id(labels, out):
+    """Largest id (> 0, else 0) of a CUDA int32 / uint16 volume into out, a [1] int32 CUDA tensor (pm_label_max_id)."""
+    check(load().pm_label_max_id(ptr(labels), _label_dtype_code(labels), labels.numel(), ptr(out), stream_ptr()),
+          "pm_label_max_id")
+    return out
+
+
+def label_overlap(labels_a, labels_b, capacity):
+    """Contingency table of two CUDA label volumes of one shape (int32 or uint16 each; pm_label_overlap) in a hash table
+    of `capacity` slots (a power of two) -> (keys [capacity] int64 = a << 32 | b, counts [capacity] int64, n_out [2]
+    int64 = (pairs written, voxels whose pair found no slot)).  The first n_out[0] entries are the table, any order;
+    n_out[1] > 0 means overflow.  Nothing is synchronised."""
+    torch = _torch()
+    if labels_a.dim() != 3 or tuple(labels_a.shape) != tuple(labels_b.shape):
+        raise ValueError("expected two 3-D volumes of one shape, got %s and %s" % (tuple(labels_a.shape),
+                                                                                   tuple(labels_b.shape)))
+    if not (labels_a.is_cuda and labels_b.is_cuda and labels_a.device == labels_b.device):
+        raise ValueError("label volumes must be CUDA tensors on the same device")
+    labels_a, labels_b = labels_a.contiguous(), labels_b.contiguous()
+    dev = labels_a.device
+    keys = torch.empty(capacity, dtype=torch.int64, device=dev)
+    counts = torch.empty(capacity, dtype=torch.int64, device=dev)
+    n_out = torch.empty(2, dtype=torch.int64, device=dev)
+    nbytes = load().pm_label_overlap_workspace_bytes(capacity)
+    ws = torch.empty(nbytes // 8 + 1, dtype=torch.int64, device=dev)
+    nz, ny, nx = labels_a.shape
+    check(load().pm_label_overlap(ptr(labels_a), _label_dtype_code(labels_a), ptr(labels_b), _label_dtype_code(labels_b),
+                                  nz, ny, nx, capacity, ptr(keys), ptr(counts), ptr(n_out), ptr(ws), nbytes, stream_ptr()),
+          "pm_label_overlap")
+    return keys, counts, n_out
+
+
 def resample_affine(src, M, out_shape, order=0, cval=0.0, out=None):
     """Volume src [sz, sy, sx] (CUDA int32, uint16 or float32 tensor) resampled into out_shape (dz, dy, dx), same dtype.
     M: 4 x 4 float64 (CUDA tensor, or host array copied over) mapping an output voxel index (z, y, x, 1) to a source
