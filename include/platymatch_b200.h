@@ -112,6 +112,30 @@ int pm_label_overlap(const void *labels_a, int dtype_a, const void *labels_b, in
 int pm_resample_affine(const void *src, int dtype, int sz, int sy, int sx, const double *M, int order, double cval,
                        void *dst, int dz, int dy, int dx, void *stream);
 
+/* ---- thin-plate spline deformation (DESIGN §8 row 8) -------------------------------------------------------------
+ * The smooth local deformation left after an affine registration: a smoothing thin-plate spline fitted to matched
+ * nuclei, and volumes warped through it.  A spline with centres y [k][3] (zyx, float64, device), coefficients
+ * c [k + 4][3] and shift_scale [6] = (shift[3], scale[3]) maps a point x to
+ *   f(x) = sum_{i<k} c_i * (-||x - y_i||) + c_k + sum_h c_{k+1+h} * (x_h - shift_h) / scale_h      (c_i = row i of c)
+ * = scipy.interpolate.RBFInterpolator(y, d, kernel='linear', degree=1, smoothing) with scipy's shift = (min + max) / 2
+ * and scale = (max - min) / 2 (0 -> 1) per axis, computed by the caller.  -||d|| is -sqrt((dz*dz + dy*dy) + dx*dx) in
+ * float64 without FMA, correctly rounded; the sum runs over the centres in ascending order, one FMA per term, so
+ * pm_spline_eval and pm_resample_spline give the same coordinate bits.  No workspace; outputs must not overlap inputs.
+ *
+ * pm_spline_system: the whole (k + 4) x (k + 4) float64 matrix [-R + smoothing I, P; P^T, 0] of the fit into lhs (row
+ *   stride ld >= k + 4): R_ij = ||y_i - y_j||, P = [1, (y - shift) / scale]; smoothing finite and >= 0.
+ * pm_spline_eval: out [n][3] = f(pts [n][3]).
+ * pm_resample_spline: the volume warp.  For output voxel x (index zyx in dst) the source coordinate is f(x); src is
+ *   sampled there exactly as pm_resample_affine does (cval outside or NaN, order 0 src[floor(c + 0.5)], order 1 clamped
+ *   trilinear, the same casts and dtypes, 64-bit offsets). */
+int pm_spline_system(const double *centres, int k, const double *shift_scale, double smoothing, double *lhs, long long ld,
+                     void *stream);
+int pm_spline_eval(const double *centres, const double *coeffs, int k, const double *shift_scale, const double *pts,
+                   long long n, double *out, void *stream);
+int pm_resample_spline(const void *src, int dtype, int sz, int sy, int sx, const double *centres, const double *coeffs,
+                       int k, const double *shift_scale, int order, double cval, void *dst, int dz, int dy, int dx,
+                       void *stream);
+
 /* ---- nuclei detection: scale-space LoG (SURVEY §2 row 10) --------------------------------------------------
  * DetectNuclei / find_spheres (platymatch/detect_nuclei/ss_log.py:25-87).  The contract is this project's own
  * (DESIGN §8 row 6; the reference's parameters are not available and agreement with it is unverified):

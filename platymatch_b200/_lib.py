@@ -38,7 +38,10 @@ SIGNATURES = {
     "pm_label_overlap_workspace_bytes": (_sz, [_u64]),
     "pm_label_overlap": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _u64, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pm_resample_affine": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _d, _vp, _i, _i, _i, _vp]),
-    "pm_detect_pass": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, ctypes.c_float, _vp, _vp]),
+    "pm_spline_system": (_i, [_vp, _i, _vp, _d, _vp, ctypes.c_longlong, _vp]),
+    "pm_spline_eval": (_i, [_vp, _vp, _i, _vp, _vp, ctypes.c_longlong, _vp, _vp]),
+    "pm_resample_spline": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _d, _vp, _i, _i, _i, _vp]),
+    "pm_detect_pass":(_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, ctypes.c_float, _vp, _vp]),
     "pm_detect_otsu_workspace_bytes": (_sz, []),
     "pm_detect_otsu": (_i, [_vp, _sz, _d, _vp, _vp, _sz, _vp]),
     "pm_detect_minima": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, ctypes.c_longlong, _vp, _vp, _vp, _vp]),

@@ -333,6 +333,69 @@ def resample_affine(src, M, out_shape, order=0, cval=0.0, out=None):
     return out
 
 
+def _spline_args(centres, coeffs, shift_scale):
+    k = centres.shape[0]
+    if centres.shape != (k, 3) or coeffs.shape != (k + 4, 3) or shift_scale.numel() != 6:
+        raise ValueError("spline arrays must be centres [k, 3], coeffs [k + 4, 3], shift_scale [6]")
+    for t in (centres, coeffs, shift_scale):
+        if not t.is_cuda or t.dtype != _torch().float64 or not t.is_contiguous():
+            raise ValueError("spline arrays must be contiguous float64 CUDA tensors")
+    return k
+
+
+def spline_system(centres, shift_scale, smoothing, out=None):
+    """The (k + 4) x (k + 4) float64 matrix [-R + smoothing I, P; P^T, 0] of a thin-plate spline fit over centres [k, 3]
+    (pm_spline_system); out: a caller-owned [k + 4, >= k + 4] float64 tensor with unit column stride."""
+    torch = _torch()
+    k = centres.shape[0]
+    if out is None:
+        out = torch.empty((k + 4, k + 4), dtype=torch.float64, device=centres.device)
+    assert out.dtype == torch.float64 and out.shape[0] == k + 4 and out.shape[1] >= k + 4 and out.stride(1) == 1
+    check(load().pm_spline_system(ptr(centres), k, ptr(shift_scale), float(smoothing), ptr(out), out.stride(0),
+                                  stream_ptr()), "pm_spline_system")
+    return out
+
+
+def spline_eval(centres, coeffs, shift_scale, pts):
+    """f(pts) [n, 3] float64 of the spline (centres [k, 3], coeffs [k + 4, 3], shift_scale [6]) at CUDA points [n, 3]
+    (pm_spline_eval)."""
+    torch = _torch()
+    k = _spline_args(centres, coeffs, shift_scale)
+    pts = pts.to(dtype=torch.float64).contiguous()
+    out = torch.empty((pts.shape[0], 3), dtype=torch.float64, device=pts.device)
+    if pts.shape[0]:
+        check(load().pm_spline_eval(ptr(centres), ptr(coeffs), k, ptr(shift_scale), ptr(pts), pts.shape[0], ptr(out),
+                                    stream_ptr()), "pm_spline_eval")
+    return out
+
+
+def resample_spline(src, centres, coeffs, shift_scale, out_shape, order=0, cval=0.0, out=None):
+    """Volume src [sz, sy, sx] (CUDA int32, uint16 or float32) warped into out_shape through a spline: output voxel x
+    samples src at f(x), as resample_affine samples at M x (pm_resample_spline).  out: a caller-owned contiguous tensor
+    of that shape and dtype."""
+    torch = _torch()
+    name = str(src.dtype).replace("torch.", "")
+    if name not in _lib.VOLUME_DTYPES:
+        raise ValueError("volume must be int32, uint16 or float32, got %s" % src.dtype)
+    if not src.is_cuda or (out is not None and (not out.is_cuda or out.device != src.device)):
+        raise ValueError("src and out must be CUDA tensors on the same device")
+    if src.dim() != 3 or len(out_shape) != 3:
+        raise ValueError("expected a 3-D volume and a 3-D output shape")
+    if order not in (0, 1):
+        raise ValueError("order must be 0 or 1, got %r" % (order,))
+    k = _spline_args(centres, coeffs, shift_scale)
+    src = src.contiguous()
+    out_shape = tuple(int(s) for s in out_shape)
+    if out is None:
+        out = torch.empty(out_shape, dtype=src.dtype, device=src.device)
+    assert out.dtype == src.dtype and tuple(out.shape) == out_shape and out.is_contiguous()
+    sz, sy, sx = src.shape
+    check(load().pm_resample_spline(ptr(src), _lib.VOLUME_DTYPES[name], sz, sy, sx, ptr(centres), ptr(coeffs), k,
+                                    ptr(shift_scale), int(order), float(cval), ptr(out), *out_shape, stream_ptr()),
+          "pm_resample_spline")
+    return out
+
+
 def cdist(a, b):
     """[n1,3], [n2,3] f64 -> [n1, ld] f32 Euclidean distances (ld = n2 rounded up to 4), as the LAP kernel wants them."""
     torch = _torch()

@@ -8,7 +8,7 @@ the registration path.  Clouds are modelled on the reference's test assets
 import numpy as np
 
 __all__ = ["make_fixed_cloud", "random_affine", "make_pair", "make_keypoints", "make_specimens", "make_label_volume",
-           "make_nuclei_image"]
+           "make_nuclei_image", "deformation_field", "make_deformed_pair"]
 
 
 def make_fixed_cloud(n, rng, filled=False):
@@ -60,6 +60,41 @@ def make_pair(n_fixed, seed=None, jitter=2.0, dropout=0.10, filled=False):
     keep = rng.permutation(keep)
     return {"moving": np.ascontiguousarray(moving_all[:, keep]), "fixed": fixed, "A_gt": a_gt,
             "gt_fixed_index": keep.astype(np.int64)}
+
+
+def deformation_field(points, field):
+    """(3, n) displacement u(p) = sum_b v_b exp(-||p - c_b||^2 / (2 sigma_b^2)) of a Gaussian-bump field
+    {"centres": (3, B), "sigma": (B,), "vectors": (3, B)} at points (3, n)."""
+    p = np.asarray(points, dtype=np.float64)
+    d2 = ((p[:, None, :] - field["centres"][:, :, None]) ** 2).sum(axis=0)          # (B, n)
+    w = np.exp(-d2 / (2.0 * field["sigma"][:, None] ** 2))
+    return field["vectors"] @ w
+
+
+def make_deformed_pair(n_fixed, seed=None, amplitude=0.03, jitter=1.0, dropout=0.10, bumps=6):
+    """A registration problem whose specimens differ by more than an affine map: `make_pair`, except that the fixed
+    cloud is first displaced by a smooth field of `bumps` Gaussian bumps before the inverse affine and the jitter, so
+    A_gt @ moving ~= fixed + u(fixed).  Each bump is centred on a random fixed nucleus, has sigma = 0.2 x the cloud's
+    largest extent E and a displacement of `amplitude` x E in a random direction at its centre.
+
+    Returns make_pair's dict plus field (as `deformation_field` takes it) and displacement = u(fixed) (3, N2).
+    """
+    rng = np.random.default_rng(n_fixed if seed is None else seed)
+    fixed = make_fixed_cloud(n_fixed, rng)
+    extent = float((fixed.max(axis=1) - fixed.min(axis=1)).max())
+    v = rng.standard_normal((3, bumps))
+    v /= np.linalg.norm(v, axis=0, keepdims=True)
+    field = {"centres": fixed[:, rng.choice(n_fixed, bumps, replace=False)].copy(),
+             "sigma": np.full(bumps, 0.2 * extent), "vectors": v * (amplitude * extent)}
+    u = deformation_field(fixed, field)
+    a_gt = random_affine(rng)
+    a_inv = np.linalg.inv(a_gt)
+    moving_all = a_inv[:3, :3] @ (fixed + u) + a_inv[:3, 3:4]
+    moving_all = moving_all + rng.normal(0.0, jitter, size=moving_all.shape)
+    keep = rng.permutation(n_fixed)[: n_fixed - int(round(dropout * n_fixed))]
+    keep = rng.permutation(keep)
+    return {"moving": np.ascontiguousarray(moving_all[:, keep]), "fixed": fixed, "A_gt": a_gt,
+            "gt_fixed_index": keep.astype(np.int64), "field": field, "displacement": u}
 
 
 def make_keypoints(pair, n_keypoints=10, seed=0, jitter=1.0):

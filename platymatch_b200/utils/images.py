@@ -4,12 +4,15 @@ SURVEY §8(f) row 5.
 
 The reference resamples through SimpleITK; here the contract is scipy.ndimage.affine_transform in voxel index space
 (order 0 or 1, mode='constant').  Agreement with the SimpleITK export itself is not verified.
+
+`transform_image_deformable` warps through the thin-plate spline of `estimate_deformation` instead of an affine map,
+with the same sampler (DESIGN §8 row 8).
 """
 import numpy as np
 
 from .. import device as D
 
-__all__ = ["transform_image"]
+__all__ = ["transform_image", "transform_image_deformable"]
 
 _DIRECT = (np.dtype(np.uint16), np.dtype(np.int32), np.dtype(np.float32))
 
@@ -27,6 +30,38 @@ def transform_image(moving_image, transform, output_shape, order=0, cval=0):
     scipy.ndimage.affine_transform(moving_image, M[:3, :3], offset=M[:3, 3], output_shape, order, mode='constant',
     cval) with M = np.linalg.inv(transform).
     """
+    a, work = _check_volume(moving_image, output_shape, order)
+    T = np.asarray(transform, dtype=np.float64)
+    if T.shape != (4, 4):
+        raise ValueError("transform must be 4 x 4, got %s" % (T.shape,))
+    M = np.linalg.inv(T)                       # output (fixed) index -> source (moving) index, as scipy takes it
+    torch = D._torch()
+    out = D.resample_affine(_upload(torch, work), torch.from_numpy(M).cuda(), output_shape, order, cval)
+    return _download(out, work, a)
+
+
+def transform_image_deformable(moving_image, deformation, output_shape, order=0, cval=0):
+    """The moving image warped into a grid of `output_shape` (the fixed image's) through a thin-plate spline, on the
+    GPU (pm_resample_spline).
+
+    deformation   the dict `estimate_deformation` returns (its `inverse` spline is used), or a Spline fixed -> moving
+    Other arguments, the dtypes and the result as `transform_image`.  For output voxel x (zyx index) the source
+    coordinate is c = inverse(x); the moving image is sampled there as `transform_image` samples it, so the result
+    equals map_coordinates(moving_image, c, order, mode='constant', cval) with c from
+    RBFInterpolator(fixed_pairs, moving_pairs, kernel='linear', degree=1, smoothing) on the grid.
+    """
+    a, work = _check_volume(moving_image, output_shape, order)
+    spline = deformation["inverse"] if isinstance(deformation, dict) else deformation
+    if not all(hasattr(spline, n) for n in ("centres", "coeffs", "shift_scale")):
+        raise ValueError("deformation must be the dict estimate_deformation returns or a Spline")
+    torch = D._torch()
+    out = D.resample_spline(_upload(torch, work), spline.centres, spline.coeffs, spline.shift_scale, output_shape,
+                            order, cval)
+    return _download(out, work, a)
+
+
+def _check_volume(moving_image, output_shape, order):
+    """(the caller's array, the uint16 / int32 / float32 array the kernels read); refused before any device work."""
     a = np.asarray(moving_image)
     if a.ndim != 3:
         raise ValueError("expected a 3-D volume, got %d-D" % a.ndim)
@@ -34,9 +69,6 @@ def transform_image(moving_image, transform, output_shape, order=0, cval=0):
         raise ValueError("output_shape must be three extents >= 1, got %r" % (output_shape,))
     if order not in (0, 1):
         raise ValueError("order must be 0 or 1, got %r" % (order,))
-    T = np.asarray(transform, dtype=np.float64)
-    if T.shape != (4, 4):
-        raise ValueError("transform must be 4 x 4, got %s" % (T.shape,))
     i32 = np.iinfo(np.int32)
     if a.dtype in _DIRECT:
         work = a
@@ -46,19 +78,23 @@ def transform_image(moving_image, transform, output_shape, order=0, cval=0):
         work = a.astype(np.int32)
     else:
         raise ValueError("volume must have an integer or float32 dtype, got %s" % a.dtype)
-    M = np.linalg.inv(T)                       # output (fixed) index -> source (moving) index, as scipy takes it
-    torch = D._torch()
-    work = np.ascontiguousarray(work)
+    return a, np.ascontiguousarray(work)
+
+
+def _upload(torch, work):
     if work.dtype == np.uint16:
-        src = torch.from_numpy(work.view(np.int16)).cuda().view(torch.uint16)
-    else:
-        src = torch.from_numpy(work).cuda()
-    out = D.resample_affine(src, torch.from_numpy(M).cuda(), output_shape, order, cval)
+        return torch.from_numpy(work.view(np.int16)).cuda().view(torch.uint16)
+    return torch.from_numpy(work).cuda()
+
+
+def _download(out, work, a):
+    torch = D._torch()
     if work.dtype == np.uint16:
         res = out.view(torch.int16).cpu().numpy().view(np.uint16)
     else:
         res = out.cpu().numpy()
     if res.dtype != a.dtype:                   # saturate into the caller's dtype, as scipy's cast does
+        i32 = np.iinfo(np.int32)
         info = np.iinfo(a.dtype)
         res = np.clip(res, max(info.min, i32.min), min(info.max, i32.max)).astype(a.dtype)
     return res
