@@ -110,10 +110,7 @@ static int pm_detect_pass_run(const float *src, int nz, int ny, int nx, const do
     const unsigned long long tiles_l = AXIS == 2 ? ((unsigned long long)nz * ny + 31) / 32
                                                  : lines_x * (unsigned long long)(AXIS == 1 ? nz : ny);
     const unsigned long long tiles = tiles_a * tiles_l;
-    if (tiles > 0x7fffffffull) {
-        pm_set_error("pm_detect_pass: volume of %d x %d x %d needs more than 2^31 - 1 CTAs", nz, ny, nx);
-        return PM_ERR_UNSUPPORTED;
-    }
+    if (int rc = pm_check_grid_1d("pm_detect_pass", "volume", tiles, nz, ny, nx)) return rc;
     const int W = PM_DT_TL + 2 * lw;
     const size_t smem = (size_t)32 * (AXIS == 2 ? (W | 1) : W) * sizeof(double);
     if (smem > 48 * 1024)
@@ -125,11 +122,6 @@ static int pm_detect_pass_run(const float *src, int nz, int ny, int nx, const do
     return PM_OK;
 }
 
-static bool pm_dt_disjoint(const void *a, size_t abytes, const void *b, size_t bbytes) {
-    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
-    return x + abytes <= y || y + bbytes <= x;
-}
-
 extern "C" int pm_detect_pass(const float *src, int nz, int ny, int nx, int axis, const double *weights, int lw,
                               const float *t0, const float *t1, float scale, float *dst, void *stream) {
     PM_REQUIRE(src && weights && dst, "null pointer");
@@ -139,9 +131,8 @@ extern "C" int pm_detect_pass(const float *src, int nz, int ny, int nx, int axis
     PM_REQUIRE(lw >= 0 && lw <= PM_DT_MAX_LW, "lw must be in [0, 384]");
     const unsigned __int128 nbytes = (unsigned __int128)nz * ny * nx * sizeof(float);
     PM_REQUIRE(nbytes < ((unsigned __int128)1 << 62), "volume too large");
-    PM_REQUIRE(pm_dt_disjoint(src, (size_t)nbytes, dst, (size_t)nbytes), "src and dst overlap (in-place is not supported)");
-    PM_REQUIRE(!t0 || (pm_dt_disjoint(t0, (size_t)nbytes, dst, (size_t)nbytes) &&
-                       pm_dt_disjoint(t1, (size_t)nbytes, dst, (size_t)nbytes)),
+    PM_REQUIRE(!pm_ranges_overlap(src, nbytes, dst, nbytes), "src and dst overlap (in-place is not supported)");
+    PM_REQUIRE(!t0 || (!pm_ranges_overlap(t0, nbytes, dst, nbytes) && !pm_ranges_overlap(t1, nbytes, dst, nbytes)),
                "t0 / t1 and dst overlap");
     const cudaStream_t s = pm_stream(stream);
     if (axis == 0) return pm_detect_pass_run<0>(src, nz, ny, nx, weights, lw, t0, t1, scale, dst, s);
@@ -333,10 +324,7 @@ extern "C" int pm_detect_minima(const float *l_prev, const float *l_cur, const f
     PM_REQUIRE(k >= 0, "k must be >= 0");
     const unsigned long long tiles_x = ((unsigned long long)nx + 31) / 32, tiles_y = ((unsigned long long)ny + 7) / 8;
     const unsigned long long tiles = tiles_x * tiles_y * (unsigned long long)nz;
-    if (tiles > 0x7fffffffull) {
-        pm_set_error("pm_detect_minima: volume of %d x %d x %d needs more than 2^31 - 1 CTAs", nz, ny, nx);
-        return PM_ERR_UNSUPPORTED;
-    }
+    if (int rc = pm_check_grid_1d(__func__, "volume", tiles, nz, ny, nx)) return rc;
     pm_detect_minima_kernel<<<(unsigned)tiles, 256, 0, pm_stream(stream)>>>(
         l_prev, l_cur, l_next, nz, ny, nx, k, threshold, (unsigned long long)capacity, keys, values, count,
         (unsigned)tiles_x, (unsigned)tiles_y);

@@ -380,17 +380,11 @@ static int pm_label_run(const T *labels, int nz, int ny, int nx, unsigned table_
     const bool stream_ok = (reinterpret_cast<size_t>(labels) & 15) == 0 && (size_t)ny * nx < ((size_t)1 << 32) &&
                            n_vox / (16 / sizeof(T)) < ((size_t)1 << 32) && !getenv("PM_LABEL_WARP_KERNEL");
     if (stream_ok) {
-        // ONE wave of resident CTAs (the kernel is a grid-stride loop): no second wave that starts ragged
         const size_t chunks = n_vox / (16 / sizeof(T));
-        static int occ_cache[64];                                  // per device (benign race: every writer stores the same value)
-        int occ = (dev >= 0 && dev < 64) ? occ_cache[dev] : 0;
-        if (occ < 1) {
-            PM_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pm_label_stream_kernel<T>, 256, 0));
-            if (occ < 1) occ = 1;
-            if (dev >= 0 && dev < 64) occ_cache[dev] = occ;
-        }
-        size_t want2 = (chunks + 256 * PM_LABEL_STREAM_HALF - 1) / (256 * PM_LABEL_STREAM_HALF);
-        const int blocks2 = (int)(want2 < (size_t)sms * occ ? (want2 ? want2 : 1) : (size_t)sms * occ);
+        const size_t want2 = (chunks + 256 * PM_LABEL_STREAM_HALF - 1) / (256 * PM_LABEL_STREAM_HALF);
+        int blocks2 = 0;
+        if (int rc = pm_resident_wave((const void *)pm_label_stream_kernel<T>, 256, dev, sms, want2, &blocks2))
+            return rc;
         pm_label_stream_kernel<T><<<blocks2, 256, 0, s>>>(labels, nz, ny, nx, table_size, acc);
     } else {
         pm_label_accumulate_kernel<T><<<blocks, 256, 0, s>>>(labels, nz, ny, nx, table_size, acc);
@@ -415,9 +409,10 @@ static int pm_label_max(const T *labels, size_t n_vox, unsigned *max_id, cudaStr
 
 extern "C" int pm_label_max_id(const void *labels, int dtype, size_t n_voxels, uint32_t *max_id, void *stream) {
     PM_REQUIRE(labels && max_id, "null pointer");
-    PM_REQUIRE(dtype == PM_LABEL_I32 || dtype == PM_LABEL_U16, "dtype must be PM_LABEL_I32 or PM_LABEL_U16");
-    if (dtype == PM_LABEL_I32) return pm_label_max((const int32_t *)labels, n_voxels, max_id, pm_stream(stream));
-    return pm_label_max((const uint16_t *)labels, n_voxels, max_id, pm_stream(stream));
+    PM_REQUIRE(pm_volume_dtype_ok(dtype, false), "dtype must be PM_LABEL_I32 or PM_LABEL_U16");
+    return pm_volume_dispatch<false>(dtype, [&](auto t) {
+        return pm_label_max((const decltype(t) *)labels, n_voxels, max_id, pm_stream(stream));
+    });
 }
 
 extern "C" size_t pm_label_workspace_bytes(uint32_t table_size) { return (size_t)table_size * 4 * sizeof(unsigned long long); }
@@ -426,7 +421,7 @@ extern "C" int pm_label_centroids(const void *labels, int dtype, int nz, int ny,
                                   double anisotropy, int capacity, int32_t *ids, double *centroids, double *sizes,
                                   int32_t *n_out, void *workspace, size_t workspace_bytes, void *stream) {
     PM_REQUIRE(labels && ids && centroids && sizes && n_out && workspace, "null pointer");
-    PM_REQUIRE(dtype == PM_LABEL_I32 || dtype == PM_LABEL_U16, "dtype must be PM_LABEL_I32 or PM_LABEL_U16");
+    PM_REQUIRE(pm_volume_dtype_ok(dtype, false), "dtype must be PM_LABEL_I32 or PM_LABEL_U16");
     PM_REQUIRE(nz >= 1 && ny >= 1 && nx >= 1 && nz < (1 << 26) && ny < (1 << 26) && nx < (1 << 26), "bad volume shape");
     PM_REQUIRE(table_size >= 1 && capacity >= 0, "bad table size / capacity");
     if (workspace_bytes < pm_label_workspace_bytes(table_size)) {
@@ -434,9 +429,8 @@ extern "C" int pm_label_centroids(const void *labels, int dtype, int nz, int ny,
         return PM_ERR_WORKSPACE;
     }
     unsigned long long *acc = (unsigned long long *)workspace;
-    if (dtype == PM_LABEL_I32)
-        return pm_label_run((const int32_t *)labels, nz, ny, nx, table_size, anisotropy, acc, capacity, ids, centroids,
-                            sizes, n_out, pm_stream(stream));
-    return pm_label_run((const uint16_t *)labels, nz, ny, nx, table_size, anisotropy, acc, capacity, ids, centroids, sizes,
-                        n_out, pm_stream(stream));
+    return pm_volume_dispatch<false>(dtype, [&](auto t) {
+        return pm_label_run((const decltype(t) *)labels, nz, ny, nx, table_size, anisotropy, acc, capacity, ids,
+                            centroids, sizes, n_out, pm_stream(stream));
+    });
 }

@@ -208,13 +208,11 @@ static int pm_overlap_run(const TA *la, const TB *lb, size_t n_vox, u64 capacity
     int dev = 0, sms = 0;
     PM_CUDA_TRY(cudaGetDevice(&dev));
     PM_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    // ONE wave of resident CTAs (the kernel is a grid-stride loop)
-    int occ = 0;
-    PM_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pm_overlap_stream_kernel<TA, TB>, 256, 0));
-    if (occ < 1) occ = 1;
     const size_t per_cta = (size_t)256 * pm_ov_half<TA, TB>();
-    const size_t want = (n_vox / 8 + per_cta - 1) / per_cta;
-    const int blocks = (int)(want < (size_t)sms * occ ? (want ? want : 1) : (size_t)sms * occ);
+    int blocks = 0;
+    if (int rc = pm_resident_wave((const void *)pm_overlap_stream_kernel<TA, TB>, 256, dev, sms,
+                                  (n_vox / 8 + per_cta - 1) / per_cta, &blocks))
+        return rc;
     pm_overlap_stream_kernel<TA, TB><<<blocks, 256, 0, s>>>(la, lb, n_vox, keys, counts, capacity - 1, dropped);
     PM_LAUNCH_CHECK();
     const u64 cwant = (capacity + 255) / 256;
@@ -228,7 +226,7 @@ extern "C" int pm_label_overlap(const void *labels_a, int dtype_a, const void *l
                                 int nx, uint64_t capacity, uint64_t *keys, uint64_t *counts, uint64_t *n_out,
                                 void *workspace, size_t workspace_bytes, void *stream) {
     PM_REQUIRE(labels_a && labels_b && keys && counts && n_out && workspace, "null pointer");
-    PM_REQUIRE((dtype_a == PM_LABEL_I32 || dtype_a == PM_LABEL_U16) && (dtype_b == PM_LABEL_I32 || dtype_b == PM_LABEL_U16),
+    PM_REQUIRE(pm_volume_dtype_ok(dtype_a, false) && pm_volume_dtype_ok(dtype_b, false),
                "dtype must be PM_LABEL_I32 or PM_LABEL_U16");
     PM_REQUIRE(nz >= 1 && ny >= 1 && nx >= 1, "every extent must be >= 1");
     PM_REQUIRE(capacity >= 1 && capacity <= ((uint64_t)1 << 58) && (capacity & (capacity - 1)) == 0,
@@ -241,13 +239,10 @@ extern "C" int pm_label_overlap(const void *labels_a, int dtype_a, const void *l
     }
     const size_t n_vox = (size_t)nz * ny * nx;
     u64 *ws = (u64 *)workspace, *ko = (u64 *)keys, *co = (u64 *)counts, *no = (u64 *)n_out;
-    cudaStream_t s = pm_stream(stream);
-    const bool a32 = dtype_a == PM_LABEL_I32, b32 = dtype_b == PM_LABEL_I32;
-    if (a32 && b32)
-        return pm_overlap_run((const int32_t *)labels_a, (const int32_t *)labels_b, n_vox, capacity, ko, co, no, ws, s);
-    if (a32)
-        return pm_overlap_run((const int32_t *)labels_a, (const uint16_t *)labels_b, n_vox, capacity, ko, co, no, ws, s);
-    if (b32)
-        return pm_overlap_run((const uint16_t *)labels_a, (const int32_t *)labels_b, n_vox, capacity, ko, co, no, ws, s);
-    return pm_overlap_run((const uint16_t *)labels_a, (const uint16_t *)labels_b, n_vox, capacity, ko, co, no, ws, s);
+    return pm_volume_dispatch<false>(dtype_a, [&](auto a) {
+        return pm_volume_dispatch<false>(dtype_b, [&](auto b) {
+            return pm_overlap_run((const decltype(a) *)labels_a, (const decltype(b) *)labels_b, n_vox, capacity, ko, co,
+                                  no, ws, pm_stream(stream));
+        });
+    });
 }

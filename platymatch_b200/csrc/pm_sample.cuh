@@ -84,9 +84,3 @@ template <typename T> __device__ __forceinline__ void pm_rs_store_quad(T *p, con
             if ((unsigned)e < left) p[e] = v[e];
     }
 }
-
-// src / dst byte ranges of the resample entry points overlap (in-place is not supported)
-static inline bool pm_ranges_overlap(const void *a, unsigned __int128 abytes, const void *b, unsigned __int128 bbytes) {
-    const unsigned __int128 a0 = (uintptr_t)a, b0 = (uintptr_t)b;
-    return !(a0 + abytes <= b0 || b0 + bbytes <= a0);
-}

@@ -179,10 +179,7 @@ static int pm_resample_spline_run(const T *src, int sz, int sy, int sx, const do
     const unsigned long long tiles_x = ((unsigned long long)dx + 4 * PM_SP_QX - 1) / (4 * PM_SP_QX);
     const unsigned long long tiles_y = ((unsigned long long)dy + PM_SP_BY - 1) / PM_SP_BY;
     const unsigned long long tiles = tiles_x * tiles_y * (unsigned long long)dz;
-    if (tiles > 0x7fffffffull) {
-        pm_set_error("pm_resample_spline: output of %d x %d x %d needs more than 2^31 - 1 CTAs", dz, dy, dx);
-        return PM_ERR_UNSUPPORTED;
-    }
+    if (int rc = pm_check_grid_1d("pm_resample_spline", "output", tiles, dz, dy, dx)) return rc;
     if (order == 0)
         pm_resample_spline_kernel<T, 0><<<(unsigned)tiles, 256, 0, s>>>(src, sz, sy, sx, centres, coeffs, k, shift_scale,
                                                                         cval, dst, dz, dy, dx, (unsigned)tiles_x,
@@ -241,26 +238,18 @@ extern "C" int pm_resample_spline(const void *src, int dtype, int sz, int sy, in
                                   const double *coeffs, int k, const double *shift_scale, int order, double cval,
                                   void *dst, int dz, int dy, int dx, void *stream) {
     PM_REQUIRE(src && centres && coeffs && shift_scale && dst, "null pointer");
-    PM_REQUIRE(dtype == PM_LABEL_I32 || dtype == PM_LABEL_U16 || dtype == PM_RESAMPLE_F32,
-               "dtype must be PM_LABEL_I32, PM_LABEL_U16 or PM_RESAMPLE_F32");
+    PM_REQUIRE(pm_volume_dtype_ok(dtype, true), "dtype must be PM_LABEL_I32, PM_LABEL_U16 or PM_RESAMPLE_F32");
     PM_REQUIRE(order == 0 || order == 1, "order must be 0 or 1");
     PM_REQUIRE(k >= 1, "k must be >= 1");
-    PM_REQUIRE(sz >= 1 && sy >= 1 && sx >= 1 && dz >= 1 && dy >= 1 && dx >= 1, "every extent must be >= 1");
-    const unsigned __int128 es = dtype == PM_LABEL_U16 ? 2 : 4;
-    const unsigned __int128 src_bytes = (unsigned __int128)sz * sy * sx * es, dst_bytes = (unsigned __int128)dz * dy * dx * es;
-    PM_REQUIRE(src_bytes < ((unsigned __int128)1 << 63) && dst_bytes < ((unsigned __int128)1 << 63), "volume too large");
-    PM_REQUIRE(!pm_ranges_overlap(src, src_bytes, dst, dst_bytes), "src and dst overlap (in-place is not supported)");
+    unsigned __int128 dst_bytes;
+    if (int rc = pm_check_volume_pair(__func__, dtype, src, sz, sy, sx, dst, dz, dy, dx, dst_bytes)) return rc;
     PM_REQUIRE(!pm_ranges_overlap(dst, dst_bytes, centres, pm_sp_centre_bytes(k)) &&
                    !pm_ranges_overlap(dst, dst_bytes, coeffs, pm_sp_coeff_bytes(k)) &&
                    !pm_ranges_overlap(dst, dst_bytes, shift_scale, 48),
                "dst overlaps the spline");
-    const cudaStream_t s = pm_stream(stream);
-    if (dtype == PM_LABEL_I32)
-        return pm_resample_spline_run((const int32_t *)src, sz, sy, sx, centres, coeffs, k, shift_scale, order, cval,
-                                      (int32_t *)dst, dz, dy, dx, s);
-    if (dtype == PM_LABEL_U16)
-        return pm_resample_spline_run((const uint16_t *)src, sz, sy, sx, centres, coeffs, k, shift_scale, order, cval,
-                                      (uint16_t *)dst, dz, dy, dx, s);
-    return pm_resample_spline_run((const float *)src, sz, sy, sx, centres, coeffs, k, shift_scale, order, cval,
-                                  (float *)dst, dz, dy, dx, s);
+    return pm_volume_dispatch<true>(dtype, [&](auto t) {
+        using T = decltype(t);
+        return pm_resample_spline_run((const T *)src, sz, sy, sx, centres, coeffs, k, shift_scale, order, cval, (T *)dst,
+                                      dz, dy, dx, pm_stream(stream));
+    });
 }

@@ -4,12 +4,16 @@ Every function here takes / returns CUDA tensors and enqueues on the current tor
 synchronises unless stated.  The reference-named numpy API (utils/, estimate_transform/) and the
 fused pipeline (pipeline.py) are built from these.
 """
+import functools
+
 import numpy as np
 
 from . import _lib
 from ._lib import NBINS, LAP_STATS, CHI2_TILE, TRANSFORMS, check, ptr, stream_ptr, load
 
 R_EDGES = np.logspace(np.log10(1 / 8), np.log10(2), 5)  # shape_context.py:24 — numpy's exact doubles
+_LABEL_DTYPES = ("int32", "uint16")                     # volumes the label kernels read
+_RESAMPLE_DTYPES = _LABEL_DTYPES + ("float32",)         # volumes the resample kernels read
 
 
 def transform_code(transform):
@@ -38,6 +42,38 @@ def to_device_points(cloud, transposed=False, device=None):
     staged = torch.empty((a.shape[0], 3), dtype=torch.float64, pin_memory=True)
     staged.numpy()[...] = a[:, :3]
     return staged.to(device or "cuda", non_blocking=True)
+
+
+def to_device_volume(a):
+    """numpy volume (uint16, int32 or float32) -> CUDA tensor of the same dtype and shape, contiguous."""
+    torch = _torch()
+    a = np.ascontiguousarray(a)
+    if a.dtype == np.uint16:                 # the bytes travel as int16, which every torch copies to the device
+        return torch.from_numpy(a.view(np.int16)).cuda().view(torch.uint16)
+    return torch.from_numpy(a).cuda()
+
+
+def to_host_volume(t):
+    """CUDA volume tensor -> numpy array of the same dtype (uint16 through int16, as to_device_volume)."""
+    torch = _torch()
+    if t.dtype == torch.uint16:
+        return t.view(torch.int16).cpu().numpy().view(np.uint16)
+    return t.cpu().numpy()
+
+
+@functools.cache
+def _dtype_codes(names):
+    torch = _torch()
+    return {getattr(torch, n): _lib.VOLUME_DTYPES[n] for n in names}
+
+
+def _dtype_code(t, names=_LABEL_DTYPES):
+    """The PM_* dtype code of a volume tensor (PM_LABEL_I32, PM_LABEL_U16, PM_RESAMPLE_F32); refused unless its dtype
+    is one of `names`."""
+    code = _dtype_codes(names).get(t.dtype)
+    if code is None:
+        raise ValueError("volume must be %s or %s, got %s" % (", ".join(names[:-1]), names[-1], t.dtype))
+    return code
 
 
 def cloud_stats(pts):
@@ -237,18 +273,11 @@ def label_centroids(labels, anisotropy=1.0, table_size=None, sync=True):
     torch = _torch()
     assert labels.dim() == 3 and labels.is_cuda
     labels = labels.contiguous()
-    if labels.dtype == torch.int32:
-        dtype = 0
-    elif labels.dtype == torch.uint16:
-        dtype = 1
-    else:
-        raise ValueError("label volume must be int32 or uint16, got %s" % labels.dtype)
+    dtype = _dtype_code(labels)
     nz, ny, nx = labels.shape
     dev = labels.device
     if table_size is None:
-        mx = torch.zeros(1, dtype=torch.int32, device=dev)
-        check(load().pm_label_max_id(ptr(labels), dtype, labels.numel(), ptr(mx), stream_ptr()), "pm_label_max_id")
-        table_size = int(mx.item()) + 1
+        table_size = int(label_max_id(labels, torch.zeros(1, dtype=torch.int32, device=dev)).item()) + 1
     cap = max(table_size - 1, 1)
     ids = torch.empty(cap, dtype=torch.int32, device=dev)
     cen = torch.empty((cap, 3), dtype=torch.float64, device=dev)
@@ -264,18 +293,9 @@ def label_centroids(labels, anisotropy=1.0, table_size=None, sync=True):
     return ids[:n], cen[:n], sizes[:n]
 
 
-def _label_dtype_code(t):
-    torch = _torch()
-    if t.dtype == torch.int32:
-        return 0
-    if t.dtype == torch.uint16:
-        return 1
-    raise ValueError("label volume must be int32 or uint16, got %s" % t.dtype)
-
-
 def label_max_id(labels, out):
     """Largest id (> 0, else 0) of a CUDA int32 / uint16 volume into out, a [1] int32 CUDA tensor (pm_label_max_id)."""
-    check(load().pm_label_max_id(ptr(labels), _label_dtype_code(labels), labels.numel(), ptr(out), stream_ptr()),
+    check(load().pm_label_max_id(ptr(labels), _dtype_code(labels), labels.numel(), ptr(out), stream_ptr()),
           "pm_label_max_id")
     return out
 
@@ -299,7 +319,7 @@ def label_overlap(labels_a, labels_b, capacity):
     nbytes = load().pm_label_overlap_workspace_bytes(capacity)
     ws = torch.empty(nbytes // 8 + 1, dtype=torch.int64, device=dev)
     nz, ny, nx = labels_a.shape
-    check(load().pm_label_overlap(ptr(labels_a), _label_dtype_code(labels_a), ptr(labels_b), _label_dtype_code(labels_b),
+    check(load().pm_label_overlap(ptr(labels_a), _dtype_code(labels_a), ptr(labels_b), _dtype_code(labels_b),
                                   nz, ny, nx, capacity, ptr(keys), ptr(counts), ptr(n_out), ptr(ws), nbytes, stream_ptr()),
           "pm_label_overlap")
     return keys, counts, n_out
@@ -312,9 +332,18 @@ def resample_affine(src, M, out_shape, order=0, cval=0.0, out=None):
     scipy.ndimage.affine_transform(src, M[:3, :3], offset=M[:3, 3], output_shape, order, mode='constant', cval)
     (pm_resample_affine).  out: a caller-owned contiguous tensor of that shape and dtype."""
     torch = _torch()
-    name = str(src.dtype).replace("torch.", "")
-    if name not in _lib.VOLUME_DTYPES:
-        raise ValueError("volume must be int32, uint16 or float32, got %s" % src.dtype)
+    src, code, out, out_shape = _resample_args(src, out_shape, order, out)
+    m = torch.as_tensor(M, dtype=torch.float64, device=src.device).reshape(16).contiguous()
+    sz, sy, sx = src.shape
+    check(load().pm_resample_affine(ptr(src), code, sz, sy, sx, ptr(m), int(order), float(cval), ptr(out), *out_shape,
+                                    stream_ptr()), "pm_resample_affine")
+    return out
+
+
+def _resample_args(src, out_shape, order, out):
+    """(contiguous src, its PM_* dtype code, out, out_shape as ints) of resample_affine / resample_spline: bad arguments
+    are refused before anything is allocated; out is allocated unless the caller gave one."""
+    code = _dtype_code(src, _RESAMPLE_DTYPES)
     if not src.is_cuda or (out is not None and (not out.is_cuda or out.device != src.device)):
         raise ValueError("src and out must be CUDA tensors on the same device")
     if src.dim() != 3 or len(out_shape) != 3:
@@ -322,15 +351,11 @@ def resample_affine(src, M, out_shape, order=0, cval=0.0, out=None):
     if order not in (0, 1):
         raise ValueError("order must be 0 or 1, got %r" % (order,))
     src = src.contiguous()
-    m = torch.as_tensor(M, dtype=torch.float64, device=src.device).reshape(16).contiguous()
     out_shape = tuple(int(s) for s in out_shape)
     if out is None:
-        out = torch.empty(out_shape, dtype=src.dtype, device=src.device)
+        out = _torch().empty(out_shape, dtype=src.dtype, device=src.device)
     assert out.dtype == src.dtype and tuple(out.shape) == out_shape and out.is_contiguous()
-    sz, sy, sx = src.shape
-    check(load().pm_resample_affine(ptr(src), _lib.VOLUME_DTYPES[name], sz, sy, sx, ptr(m), int(order), float(cval),
-                                    ptr(out), *out_shape, stream_ptr()), "pm_resample_affine")
-    return out
+    return src, code, out, out_shape
 
 
 def _spline_args(centres, coeffs, shift_scale):
@@ -373,26 +398,12 @@ def resample_spline(src, centres, coeffs, shift_scale, out_shape, order=0, cval=
     """Volume src [sz, sy, sx] (CUDA int32, uint16 or float32) warped into out_shape through a spline: output voxel x
     samples src at f(x), as resample_affine samples at M x (pm_resample_spline).  out: a caller-owned contiguous tensor
     of that shape and dtype."""
-    torch = _torch()
-    name = str(src.dtype).replace("torch.", "")
-    if name not in _lib.VOLUME_DTYPES:
-        raise ValueError("volume must be int32, uint16 or float32, got %s" % src.dtype)
-    if not src.is_cuda or (out is not None and (not out.is_cuda or out.device != src.device)):
-        raise ValueError("src and out must be CUDA tensors on the same device")
-    if src.dim() != 3 or len(out_shape) != 3:
-        raise ValueError("expected a 3-D volume and a 3-D output shape")
-    if order not in (0, 1):
-        raise ValueError("order must be 0 or 1, got %r" % (order,))
+    _torch()
     k = _spline_args(centres, coeffs, shift_scale)
-    src = src.contiguous()
-    out_shape = tuple(int(s) for s in out_shape)
-    if out is None:
-        out = torch.empty(out_shape, dtype=src.dtype, device=src.device)
-    assert out.dtype == src.dtype and tuple(out.shape) == out_shape and out.is_contiguous()
+    src, code, out, out_shape = _resample_args(src, out_shape, order, out)
     sz, sy, sx = src.shape
-    check(load().pm_resample_spline(ptr(src), _lib.VOLUME_DTYPES[name], sz, sy, sx, ptr(centres), ptr(coeffs), k,
-                                    ptr(shift_scale), int(order), float(cval), ptr(out), *out_shape, stream_ptr()),
-          "pm_resample_spline")
+    check(load().pm_resample_spline(ptr(src), code, sz, sy, sx, ptr(centres), ptr(coeffs), k, ptr(shift_scale),
+                                    int(order), float(cval), ptr(out), *out_shape, stream_ptr()), "pm_resample_spline")
     return out
 
 

@@ -12,25 +12,11 @@ Without keypoints, two label volumes (e.g. the fixed segmentation and the moving
 import numpy as np
 
 from . import device as D
+from .utils.labels import _check_label_volume
 
 __all__ = ["assign_by_distance", "calculate_metrics", "label_contingency", "match_labels"]
 
-_ID_MAX = 2 ** 31 - 1
 LAP_MAX_COLUMNS = 24576          # the assignment kernel's limit (pm_lap_solve refuses wider matrices)
-
-
-def _check_label_volume(a, name):
-    """A host label volume as the int32 / uint16 array the table pass reads; refused before any device work."""
-    a = np.asarray(a)
-    if a.ndim != 3:
-        raise ValueError("%s: expected a 3-D label volume, got %d-D" % (name, a.ndim))
-    if not np.issubdtype(a.dtype, np.integer):
-        raise ValueError("%s: label volumes must have an integer dtype, got %s" % (name, a.dtype))
-    if a.dtype in (np.dtype(np.int32), np.dtype(np.uint16)):
-        return np.ascontiguousarray(a)
-    if a.size and a.max() > _ID_MAX:
-        raise ValueError("%s: ids above 2^31 - 1 are not supported (largest is %d)" % (name, int(a.max())))
-    return np.ascontiguousarray(np.maximum(a, 0).astype(np.int32))          # (ids <= 0 are background)
 
 
 def _check_pair(labels_a, labels_b):
@@ -38,12 +24,6 @@ def _check_pair(labels_a, labels_b):
     if a.shape != b.shape:
         raise ValueError("label volumes differ in shape: %s and %s" % (a.shape, b.shape))
     return a, b
-
-
-def _to_device(torch, a):
-    if a.dtype == np.uint16:
-        return torch.from_numpy(a.view(np.int16)).cuda().view(torch.uint16)
-    return torch.from_numpy(a).cuda()
 
 
 def _pow2(n):
@@ -63,7 +43,7 @@ def _contingency(a, b):
     Host synchronisations: 5 (the upload of each volume from pageable memory, the largest ids, the pair count, the
     result copy), plus 1 per overflow rerun."""
     torch = D._torch()
-    ta, tb = _to_device(torch, a), _to_device(torch, b)
+    ta, tb = D.to_device_volume(a), D.to_device_volume(b)
     mx = torch.zeros(2, dtype=torch.int32, device=ta.device)
     D.label_max_id(ta, mx[0:1])
     D.label_max_id(tb, mx[1:2])

@@ -35,9 +35,8 @@ def transform_image(moving_image, transform, output_shape, order=0, cval=0):
     if T.shape != (4, 4):
         raise ValueError("transform must be 4 x 4, got %s" % (T.shape,))
     M = np.linalg.inv(T)                       # output (fixed) index -> source (moving) index, as scipy takes it
-    torch = D._torch()
-    out = D.resample_affine(_upload(torch, work), torch.from_numpy(M).cuda(), output_shape, order, cval)
-    return _download(out, work, a)
+    out = D.resample_affine(D.to_device_volume(work), M, output_shape, order, cval)
+    return _download(out, a)
 
 
 def transform_image_deformable(moving_image, deformation, output_shape, order=0, cval=0):
@@ -54,10 +53,9 @@ def transform_image_deformable(moving_image, deformation, output_shape, order=0,
     spline = deformation["inverse"] if isinstance(deformation, dict) else deformation
     if not all(hasattr(spline, n) for n in ("centres", "coeffs", "shift_scale")):
         raise ValueError("deformation must be the dict estimate_deformation returns or a Spline")
-    torch = D._torch()
-    out = D.resample_spline(_upload(torch, work), spline.centres, spline.coeffs, spline.shift_scale, output_shape,
+    out = D.resample_spline(D.to_device_volume(work), spline.centres, spline.coeffs, spline.shift_scale, output_shape,
                             order, cval)
-    return _download(out, work, a)
+    return _download(out, a)
 
 
 def _check_volume(moving_image, output_shape, order):
@@ -81,18 +79,9 @@ def _check_volume(moving_image, output_shape, order):
     return a, np.ascontiguousarray(work)
 
 
-def _upload(torch, work):
-    if work.dtype == np.uint16:
-        return torch.from_numpy(work.view(np.int16)).cuda().view(torch.uint16)
-    return torch.from_numpy(work).cuda()
-
-
-def _download(out, work, a):
-    torch = D._torch()
-    if work.dtype == np.uint16:
-        res = out.view(torch.int16).cpu().numpy().view(np.uint16)
-    else:
-        res = out.cpu().numpy()
+def _download(out, a):
+    """The resampled volume as a numpy array of the caller's dtype."""
+    res = D.to_host_volume(out)
     if res.dtype != a.dtype:                   # saturate into the caller's dtype, as scipy's cast does
         i32 = np.iinfo(np.int32)
         info = np.iinfo(a.dtype)

@@ -19,20 +19,6 @@ pytestmark = pytest.mark.gpu
 NEAR = 1e-6                 # oracle coordinates this close to a rounding or domain boundary may round either way
 
 
-def _to_device(a):
-    import torch
-    if a.dtype == np.uint16:
-        return torch.from_numpy(np.ascontiguousarray(a).view(np.int16)).cuda().view(torch.uint16)
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
-def _to_host(t):
-    import torch
-    if t.dtype == torch.uint16:
-        return t.view(torch.int16).cpu().numpy().view(np.uint16)
-    return t.cpu().numpy()
-
-
 def _shell(k, seed):
     """k nuclei-like centres (3, k) of a make_fixed_cloud shell and a smooth displacement of them as the targets."""
     from platymatch_b200.synthetic import make_deformed_pair
@@ -145,15 +131,17 @@ def _near_boundary(c, shape):
 @pytest.mark.parametrize("case", CASES)
 def test_warp_matches_scipy_oracle(case, dtype, order):
     import scipy.ndimage as nd
+    import torch
     from platymatch_b200 import device as D
     from platymatch_b200.estimate_transform.deformable import fit_spline
     sshape, oshape, y, t, lam, cval = _spline_case(case)
     src = _source(sshape, dtype, seed=len(case) + order)
     sp = fit_spline(y, t, smoothing=lam)
-    out = _to_host(D.resample_spline(_to_device(src), sp.centres, sp.coeffs, sp.shift_scale, oshape, order, cval))
+    out = D.to_host_volume(D.resample_spline(D.to_device_volume(src), sp.centres, sp.coeffs, sp.shift_scale, oshape,
+                                             order, cval))
     g = SO.grid(oshape)
     c_ref = SO.rbf(y, t, lam)(g).T                                            # the oracle's coordinates
-    c_gpu = D.spline_eval(sp.centres, sp.coeffs, sp.shift_scale, _to_device(g)).cpu().numpy().T
+    c_gpu = D.spline_eval(sp.centres, sp.coeffs, sp.shift_scale, torch.from_numpy(g).cuda()).cpu().numpy().T
     assert np.abs(c_gpu - c_ref).max() <= 1e-7
     ref = nd.map_coordinates(src, c_ref, order=order, mode="constant", cval=cval).reshape(oshape)
     near = _near_boundary(c_ref, sshape).reshape(oshape)
@@ -186,14 +174,16 @@ def test_warp_matches_scipy_oracle(case, dtype, order):
 def test_warp_samples_at_eval_coordinates(dtype):
     """pm_spline_eval on every voxel gives the coordinates: the numpy order-0 sampler at them equals pm_resample_spline
     bit for bit (no boundary exception: the two kernels share the evaluation routine)."""
+    import torch
     from platymatch_b200 import device as D
     from platymatch_b200.estimate_transform.deformable import fit_spline
     sshape, oshape, y, t, lam, cval = _spline_case("k400_larger_out")
     oshape = (13, 37, 45)
     sp = fit_spline(y, t, smoothing=lam)
     src = _source(sshape, dtype, seed=3)
-    out = _to_host(D.resample_spline(_to_device(src), sp.centres, sp.coeffs, sp.shift_scale, oshape, 0, -2.0))
-    c = D.spline_eval(sp.centres, sp.coeffs, sp.shift_scale, _to_device(SO.grid(oshape))).cpu().numpy().T
+    out = D.to_host_volume(D.resample_spline(D.to_device_volume(src), sp.centres, sp.coeffs, sp.shift_scale, oshape,
+                                             0, -2.0))
+    c = D.spline_eval(sp.centres, sp.coeffs, sp.shift_scale, torch.from_numpy(SO.grid(oshape)).cuda()).cpu().numpy().T
     want = SO.sample_order0(src, c, -2.0).reshape(oshape)
     assert np.array_equal(out.view(np.uint8), want.view(np.uint8))
     assert np.count_nonzero(want != np.asarray(-2.0).astype(dtype)) > want.size // 2
@@ -221,7 +211,7 @@ def test_warp_beyond_2_31_voxels():
     scale = (np.array(sshape, dtype=np.float64) - 1.5) / (np.array(oshape) - 1)
     t = y * scale[:, None] + 0.3 + rng.normal(0, 0.5, size=y.shape)
     sp = fit_spline(y, t, smoothing=0.0)
-    out = _to_host(D.resample_spline(src, sp.centres, sp.coeffs, sp.shift_scale, oshape, 0, -1.0))
+    out = D.to_host_volume(D.resample_spline(src, sp.centres, sp.coeffs, sp.shift_scale, oshape, 0, -1.0))
     del src
     torch.cuda.empty_cache()
     flat = rng.choice(out.size, 100000, replace=False)
@@ -241,7 +231,7 @@ def test_warp_on_side_stream():
     from platymatch_b200 import device as D
     from platymatch_b200.estimate_transform.deformable import fit_spline
     sshape, oshape, y, t, lam, cval = _spline_case("k400_smaller_out")
-    src = _to_device(_source(sshape, np.float32, seed=9))
+    src = D.to_device_volume(_source(sshape, np.float32, seed=9))
     torch.cuda.synchronize()
     side = torch.cuda.Stream()
     with torch.cuda.stream(side):
@@ -250,7 +240,7 @@ def test_warp_on_side_stream():
     side.synchronize()
     sp0 = fit_spline(y, t, smoothing=lam)
     ref = D.resample_spline(src, sp0.centres, sp0.coeffs, sp0.shift_scale, oshape, 1, cval)
-    assert np.array_equal(_to_host(got).view(np.uint32), _to_host(ref).view(np.uint32))
+    assert np.array_equal(D.to_host_volume(got).view(np.uint32), D.to_host_volume(ref).view(np.uint32))
 
 
 def _held_out_errors(moving, fixed, gt, T, held, smoothing):

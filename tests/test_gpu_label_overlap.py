@@ -187,9 +187,7 @@ def test_table_overflow_reruns(monkeypatch):
     ia, _, _ = assert_table(a, b)
     assert ia.size > 30000 and len(calls) >= 3 and calls[0] == 2048, calls
     # the device call reports the overflow itself: pairs written <= capacity, dropped voxels > 0
-    torch = D._torch()
-    keys, counts, n_out = real(torch.from_numpy(a).cuda(), torch.from_numpy(b.view(np.int16)).cuda().view(torch.uint16),
-                               1024)
+    keys, counts, n_out = real(D.to_device_volume(a), D.to_device_volume(b), 1024)
     n_pairs, dropped = n_out.cpu().tolist()
     assert n_pairs <= 1024 and dropped > 0
     assert int(counts[:n_pairs].sum()) + dropped == np.count_nonzero((a > 0) | (b > 0))

@@ -20,26 +20,12 @@ def _scipy(src, M, shape, order, cval):
                                cval=cval)
 
 
-def _to_device(a):
-    import torch
-    if a.dtype == np.uint16:
-        return torch.from_numpy(np.ascontiguousarray(a).view(np.int16)).cuda().view(torch.uint16)
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
-def _to_host(t):
-    import torch
-    if t.dtype == torch.uint16:
-        return t.view(torch.int16).cpu().numpy().view(np.uint16)
-    return t.cpu().numpy()
-
-
 def _gpu(src, M, shape, order, cval):
     import torch
     from platymatch_b200 import device as D
-    out = D.resample_affine(_to_device(src), torch.from_numpy(np.ascontiguousarray(M, dtype=np.float64)).cuda(), shape,
-                            order, cval)
-    return _to_host(out)
+    out = D.resample_affine(D.to_device_volume(src), torch.from_numpy(np.ascontiguousarray(M, dtype=np.float64)).cuda(),
+                            shape, order, cval)
+    return D.to_host_volume(out)
 
 
 def _rotation(angles):
@@ -159,7 +145,7 @@ def test_resample_unaligned_and_out_buffer():
     ref = _scipy(src, M, (7, 11, 21), 0, 0.0)
     big = torch.zeros(7 * 11 * 21 + 1, dtype=torch.int32, device="cuda")
     out = big[1:].view(7, 11, 21)
-    res = D.resample_affine(_to_device(src), torch.from_numpy(M).cuda(), (7, 11, 21), 0, 0.0, out=out)
+    res = D.resample_affine(D.to_device_volume(src), torch.from_numpy(M).cuda(), (7, 11, 21), 0, 0.0, out=out)
     assert res.data_ptr() == out.data_ptr()
     assert np.array_equal(out.cpu().numpy(), ref) and int(big[0]) == 0
 
@@ -180,7 +166,7 @@ def test_resample_beyond_2_31_voxels():
     oshape = (128, 64, 65)
     lin3 = _rotation([0.01, -0.008, 0.012]) @ np.diag([2047 / 128, 1023 / 64, 1039 / 65])
     M = _affine(lin3, [3.0, 2.5, 1.0])
-    out = _to_host(D.resample_affine(src, torch.from_numpy(M).cuda(), oshape, 0, -1.0))
+    out = D.to_host_volume(D.resample_affine(src, torch.from_numpy(M).cuda(), oshape, 0, -1.0))
     del src
     torch.cuda.empty_cache()
     rng = np.random.default_rng(0)
@@ -281,7 +267,7 @@ def test_resample_on_side_stream_after_registration():
     from platymatch_b200.synthetic import make_pair
     pair = make_pair(600, seed=11)
     vol = _source((64, 80, 96), np.float32, seed=9)
-    dev_vol = _to_device(vol)
+    dev_vol = D.to_device_volume(vol)
     centre = torch.tensor([31.5, 39.5, 47.5], dtype=torch.float64, device="cuda")
     torch.cuda.synchronize()
     side = torch.cuda.Stream()
@@ -293,8 +279,8 @@ def test_resample_on_side_stream_after_registration():
         m[:3, 3] = centre - m[:3, :3] @ centre
         out = D.resample_affine(dev_vol, m, (70, 75, 90), 1, -1.0)
     side.synchronize()
-    got = _to_host(out)
-    ref = _to_host(D.resample_affine(dev_vol, m, (70, 75, 90), 1, -1.0))
+    got = D.to_host_volume(out)
+    ref = D.to_host_volume(D.resample_affine(dev_vol, m, (70, 75, 90), 1, -1.0))
     assert np.array_equal(got.view(np.uint32), ref.view(np.uint32))
     assert np.count_nonzero(ref != -1.0) > ref.size // 3           # (0.68 of the grid maps inside with A_gt)
 

@@ -72,6 +72,20 @@ def test_label_volumes_refused_before_device(pair, monkeypatch):
         match_labels(a, b)
 
 
+BAD_VOLUMES = [np.zeros((4, 5), np.int32), np.zeros((2, 4, 5, 1), np.uint16), np.zeros((2, 4, 5), np.float32),
+               np.zeros((2, 4, 5), np.bool_), np.full((2, 4, 5), 2 ** 31, np.int64),
+               np.full((2, 4, 5), 2 ** 32 - 1, np.uint32)]
+
+
+@pytest.mark.parametrize("vol", range(len(BAD_VOLUMES)))
+def test_detections_from_labels_refused_before_device(vol, monkeypatch):
+    """detections_from_labels follows the label-volume policy of the table pass, checked before any device work."""
+    from platymatch_b200.utils.labels import detections_from_labels
+    _no_device(monkeypatch)
+    with pytest.raises(ValueError):
+        detections_from_labels(BAD_VOLUMES[vol])
+
+
 @pytest.mark.parametrize("thresholds", [(0.0,), (1.5,), (-0.1,), (0.5, float("nan")), (), (0.5, 1.0000001)])
 def test_thresholds_refused_before_device(thresholds, monkeypatch):
     from platymatch_b200.evaluate_metrics import match_labels
@@ -83,7 +97,7 @@ def test_thresholds_refused_before_device(thresholds, monkeypatch):
 
 def test_other_integer_dtypes_go_through_int32():
     """int64 / int8 / uint32 volumes within range become int32 with ids <= 0 as background; no device involved."""
-    from platymatch_b200.evaluate_metrics import _check_label_volume
+    from platymatch_b200.utils.labels import _check_label_volume
     a = np.array([[[-(2 ** 40), -1, 0, 5, 2 ** 31 - 1]]], dtype=np.int64)
     got = _check_label_volume(a, "a")
     assert got.dtype == np.int32 and got.tolist() == [[[0, 0, 0, 5, 2 ** 31 - 1]]]

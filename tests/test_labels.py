@@ -98,9 +98,14 @@ def test_detections_from_labels_int64_and_negative_background():
     from platymatch_b200.utils.labels import detections_from_labels
     rng = np.random.default_rng(3)
     vol = rng.integers(0, 6, size=(9, 10, 11)).astype(np.int64)
-    det, sizes, ids = detections_from_labels(vol)
-    rdet, rsizes, rids = O.detections_from_labels(vol)
-    assert np.array_equal(ids, rids) and np.array_equal(det, rdet) and np.array_equal(sizes, rsizes)
+    neg = vol.copy()
+    neg[0, 0, :] = -(2 ** 32) + 5            # below -2^31: background, not id 5 after a wrapping cast to int32
+    neg[4, :, 3] = -1
+    for v in (vol, neg):
+        det, sizes, ids = detections_from_labels(v)
+        rdet, rsizes, rids = O.detections_from_labels(np.maximum(v, 0))    # (the oracle keeps negative ids)
+        assert ids.dtype == np.int64
+        assert np.array_equal(ids, rids) and np.array_equal(det, rdet) and np.array_equal(sizes, rsizes)
     with pytest.raises(ValueError):
         detections_from_labels(vol.astype(np.float32))
 

@@ -38,7 +38,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
-from resample_bench import SHAPE, near_rigid, to_device                 # noqa: E402
+from resample_bench import SHAPE, near_rigid                            # noqa: E402
 
 N = 6000
 SUB = (8, 64, 128)
@@ -179,7 +179,7 @@ def main():
         clock_hz = None
     warps = {}
     for name, vol, order in (("int32_order0", labels, 0), ("float32_order1", intensity, 1)):
-        sv = to_device(torch, vol)
+        sv = D.to_device_volume(vol)
         o = torch.empty(SHAPE, dtype=sv.dtype, device="cuda")
         t = events_ms(torch, lambda: D.resample_spline(sv, sp.centres, sp.coeffs, sp.shift_scale, SHAPE, order, 0.0,
                                                        out=o), warmup=1, reps=3)

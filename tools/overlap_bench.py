@@ -95,7 +95,7 @@ def main():
     peak = copy_gbs(torch)
     rows = []
     for name, b in (("int32_int32", warped32), ("int32_uint16", warped16)):
-        ta, tb = E._to_device(torch, fixed), E._to_device(torch, b)
+        ta, tb = D.to_device_volume(fixed), D.to_device_volume(b)
         mx = torch.zeros(2, dtype=torch.int32, device="cuda")
         D.label_max_id(ta, mx[0:1])
         D.label_max_id(tb, mx[1:2])

@@ -66,12 +66,6 @@ def near_rigid():
     return T
 
 
-def to_device(torch, a):
-    if a.dtype == np.uint16:
-        return torch.from_numpy(a.view(np.int16)).cuda().view(torch.uint16)
-    return torch.from_numpy(a).cuda()
-
-
 def time_ms(torch, fn, flush, warmup=3, reps=10):
     for _ in range(warmup):
         fn()
@@ -99,7 +93,7 @@ def copy_gbs(torch, flush, nbytes=1 << 30):
 def measure(torch, D, vols, flush, peak, transforms=("identity", "near_rigid")):
     rows = []
     for name, vol, order in vols:
-        src = to_device(torch, vol)
+        src = D.to_device_volume(vol)
         out = torch.empty_like(src)
         nbytes = 2 * vol.nbytes
         for tname in transforms:
@@ -121,8 +115,8 @@ def cpu_baseline(torch, D, vols, rows):
         ref = nd.affine_transform(vol, M[:3, :3], offset=M[:3, 3], output_shape=SHAPE, order=order, mode="constant",
                                   cval=0.0)
         t = time.perf_counter() - t0
-        got = D.resample_affine(to_device(torch, vol), torch.from_numpy(M).cuda(), SHAPE, order, 0.0)
-        got = (got.view(torch.int16).cpu().numpy().view(np.uint16) if vol.dtype == np.uint16 else got.cpu().numpy())
+        got = D.resample_affine(D.to_device_volume(vol), torch.from_numpy(M).cuda(), SHAPE, order, 0.0)
+        got = D.to_host_volume(got)
         diff = int(np.count_nonzero(got != ref))
         gpu = next(r for r in rows if r["workload"] == name and r["transform"] == "near_rigid")
         gpu["cpu_baseline"] = {"seconds": t, "voxels_per_s": vol.size / t, "cores": 1,
