@@ -209,7 +209,8 @@ int pm_shape_context_hist_rows(const double *pts, int n, const double *centroid,
 /* ---- K3  chi^2 histogram-distance cost matrix ---------------------------------------------------
  * get_unary_distance (shape_context.py:88-99) over all pairs (_dock_widget.py:547-602):
  * cost[i][j] = 0.5 * sum_k (a_ik - b_jk)^2 / (a_ik + b_jk), equal bins skipped.  Packed FP32,
- * register tiled, two bins per reciprocal, structurally empty bins skipped per 128 x 128 tile.
+ * register tiled, two bins per reciprocal, structurally empty bins skipped per warp (16 rows x 128
+ * columns).
  *
  * pm_chi2_operand prepares one cloud's histograms for either side of the matrix:
  *   out   [361][ld] float32 bin-major, ld = n rounded up to 128: count / row total (one rounding);
@@ -217,13 +218,15 @@ int pm_shape_context_hist_rows(const double *pts, int n, const double *centroid,
  *         makes equal-and-empty bins contribute exactly 0 without a branch
  *   mask  [ld/128][12] uint32: bit k of block q = some histogram in rows [128q, 128q+128) has a
  *         non-empty bin k
+ *   fine  [ld/16][12] uint32: the same per block of 16 rows
  * pm_chi2_cost writes rows [row_begin,row_end) of the n1 x n2 matrix to cost + (i - row_begin) * ldc
- * (row sharding across GPUs: each rank passes its own 128-aligned range and buffer). */
+ * (row sharding across GPUs: each rank passes its own 128-aligned range and buffer).  a_fine is the row
+ * side's fine mask, b_mask the column side's 128-block mask. */
 #define PM_CHI2_EPS 8.673617379884035e-19f
-int pm_chi2_operand(const uint32_t *counts, int n, float *out, int ld, uint32_t *mask, void *stream);
+int pm_chi2_operand(const uint32_t *counts, int n, float *out, int ld, uint32_t *mask, uint32_t *fine, void *stream);
 /* same from already-normalised float32 histograms [n][360] (values <= 0 count as empty) */
-int pm_chi2_operand_f32(const float *hist, int n, float *out, int ld, uint32_t *mask, void *stream);
-int pm_chi2_cost(const float *a_t, int lda, const uint32_t *a_mask, int n1, const float *b_t, int ldb,
+int pm_chi2_operand_f32(const float *hist, int n, float *out, int ld, uint32_t *mask, uint32_t *fine, void *stream);
+int pm_chi2_cost(const float *a_t, int lda, const uint32_t *a_fine, int n1, const float *b_t, int ldb,
                  const uint32_t *b_mask, int n2, int row_begin, int row_end, float *cost, int ldc, void *stream);
 
 /* ---- K4  linear sum assignment ------------------------------------------------------------------

@@ -52,8 +52,8 @@ SIGNATURES = {
     "pm_mean_distance_workspace_bytes": (_sz, [_i]),
     "pm_mean_distance": (_i, [_vp, _i, _vp, _vp, _sz, _vp]),
     "pm_shape_context_hist_rows": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
-    "pm_chi2_operand": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
-    "pm_chi2_operand_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
+    "pm_chi2_operand": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp]),
+    "pm_chi2_operand_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp]),
     "pm_chi2_cost": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _i, _vp]),
     "pm_lap_workspace_bytes": (_sz, [_i, _i, _i]),
     "pm_lap_solve": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),

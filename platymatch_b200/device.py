@@ -118,10 +118,11 @@ def padded(n, tile=CHI2_TILE):
 
 class Chi2Operand:
     """One side of the chi^2 cost kernel: bin-major float32 histograms [361, ld] (empty bins = 2^-60, row
-    360 = null bin) and the per-128-block non-empty-bin masks [ld/128, 12] (see pm_chi2_operand)."""
+    360 = null bin), the per-128-block non-empty-bin masks [ld/128, 12] and the same per 16-block `fine`
+    [ld/16, 12] (see pm_chi2_operand)."""
 
-    def __init__(self, t, mask, n):
-        self.t, self.mask, self.n, self.ld = t, mask, n, t.shape[1]
+    def __init__(self, t, mask, fine, n):
+        self.t, self.mask, self.fine, self.n, self.ld = t, mask, fine, n, t.shape[1]
 
 
 def chi2_operand(hist_2d):
@@ -131,13 +132,15 @@ def chi2_operand(hist_2d):
     ld = padded(n)
     out = torch.empty((NBINS + 1, ld), dtype=torch.float32, device=hist_2d.device)
     mask = torch.empty((ld // CHI2_TILE, 12), dtype=torch.int32, device=hist_2d.device)
+    fine = torch.empty((ld // 16, 12), dtype=torch.int32, device=hist_2d.device)
     hist_2d = hist_2d.contiguous()
     if hist_2d.dtype == torch.float32:
-        check(load().pm_chi2_operand_f32(ptr(hist_2d), n, ptr(out), ld, ptr(mask), stream_ptr()), "pm_chi2_operand_f32")
+        check(load().pm_chi2_operand_f32(ptr(hist_2d), n, ptr(out), ld, ptr(mask), ptr(fine), stream_ptr()),
+              "pm_chi2_operand_f32")
     else:
         assert hist_2d.dtype in (torch.int32, torch.uint32)
-        check(load().pm_chi2_operand(ptr(hist_2d), n, ptr(out), ld, ptr(mask), stream_ptr()), "pm_chi2_operand")
-    return Chi2Operand(out, mask, n)
+        check(load().pm_chi2_operand(ptr(hist_2d), n, ptr(out), ld, ptr(mask), ptr(fine), stream_ptr()), "pm_chi2_operand")
+    return Chi2Operand(out, mask, fine, n)
 
 
 def chi2_cost(a, b, out=None, row_begin=0, row_end=None, out_ptr=None, out_ld=None):
@@ -150,14 +153,14 @@ def chi2_cost(a, b, out=None, row_begin=0, row_end=None, out_ptr=None, out_ld=No
     ldc = (n2 + 3) // 4 * 4
     if out_ptr is not None:
         import ctypes
-        check(load().pm_chi2_cost(ptr(a.t), a.ld, ptr(a.mask), n1, ptr(b.t), b.ld, ptr(b.mask), n2, row_begin, row_end,
+        check(load().pm_chi2_cost(ptr(a.t), a.ld, ptr(a.fine), n1, ptr(b.t), b.ld, ptr(b.mask), n2, row_begin, row_end,
                                   ctypes.c_void_p(int(out_ptr)), int(out_ld if out_ld is not None else ldc), stream_ptr()),
               "pm_chi2_cost")
         return None
     if out is None:
         out = torch.empty((row_end - row_begin, ldc), dtype=torch.float32, device=a.t.device)
     assert out.stride(-1) == 1 and out.shape[-1] >= n2
-    check(load().pm_chi2_cost(ptr(a.t), a.ld, ptr(a.mask), n1, ptr(b.t), b.ld, ptr(b.mask), n2, row_begin, row_end,
+    check(load().pm_chi2_cost(ptr(a.t), a.ld, ptr(a.fine), n1, ptr(b.t), b.ld, ptr(b.mask), n2, row_begin, row_end,
                               ptr(out), out.stride(-2), stream_ptr()), "pm_chi2_cost")
     return out
 
