@@ -34,7 +34,9 @@ def detections_from_labels(label_image, anisotropy=1.0):
       detections  (3, N) float64, rows z, y, x = np.mean of the voxel indices of each id (:506-507,520-521)
       sizes       (N,)  float64 = anisotropy * voxel count (:508,517)
       ids         (N,)  the positive ids in np.unique order (:497-500), in label_image's dtype
-    One streaming pass on the GPU instead of one np.where pass per id.
+    One streaming pass on the GPU instead of one np.where pass per id.  Sparse ids are fine at any volume size: when
+    a table with one entry per possible id would cost more than the volume warrants, the ids are compacted on the GPU
+    first (device.label_centroids), at 4 bytes per voxel of temporary device memory plus at most 343 MB of scratch.
     """
     a = np.asarray(label_image)
     work = _check_label_volume(a, "label_image")
